@@ -21,6 +21,8 @@
  *    the reference's cap t = min(num_remove, n_g - 1) (preconditioner.cc:358,723,846).
  *    n_graphs = 1 with graph_ptr = {0, n} is the reference's semantics (a PyG batch treated as
  *    one graph, scripts/graph_shared.py:139-146).
+ *  - Which vertices survive can also be named: rlap_schur_eliminate_keep takes a keep mask (protected vertices are
+ *    never eliminated), which turns full-clique mode into an exact Kron reduction onto any terminal set.
  */
 #ifndef RLAP_B200_H
 #define RLAP_B200_H
@@ -54,8 +56,9 @@ enum {
     RLAP_FLAG_FULL_CLIQUE = 1,   /* replace sampling by full clique elimination: exact Schur complement */
     RLAP_FLAG_SHARED_ORDER = 2,  /* o_v=random: all views share view 0's vertex permutation              */
     RLAP_FLAG_NO_VALIDATE = 4,   /* rlap_ingest: skip the symmetry check                                 */
-    RLAP_FLAG_CHECK_LIVE = 8     /* self-check: count the surviving vertices whose emitted entry count differs
+    RLAP_FLAG_CHECK_LIVE = 8,    /* self-check: count the surviving vertices whose emitted entry count differs
                                     from the live counter the elimination maintained (stats[15], must be 0)  */
+    RLAP_FLAG_KEEP = 16          /* rlap_schur_workspace_bytes: room for a keep mask (rlap_schur_eliminate_keep) */
 };
 
 const char* rlap_status_string(int status);
@@ -99,6 +102,21 @@ int rlap_schur_eliminate(int64_t n, int64_t nnz, const int32_t* csr_ptr, const i
  * [9..14] time inside the elimination kernel (us): init, min-key scan, candidate selection, truncation,
  * warp-level elimination, block-level elimination; [15] (only with RLAP_FLAG_CHECK_LIVE) number of
  * surviving vertices whose scattered entry count differs from their live counter: must be 0. */
+
+/* ---- views onto a caller-chosen vertex set (no reference counterpart: the reference only takes a count) ----------
+ * rlap_schur_eliminate with one more argument: keep, device uint8[n] or NULL. A nonzero keep[v] protects v: it is
+ * never eliminated, in every view of the call. For graph g with m_g unprotected vertices the cap becomes
+ * t_g = min(max(num_remove[g], 0), m_g) when g has a protected vertex (every unprotected vertex may go) and stays
+ * min(max(num_remove[g], 0), n_g - 1) otherwise. o_v = random ranks the unprotected vertices of g (numbered by ascending
+ * id) with the same keyed permutation over m_g; degree / coarsen take the minimum key, the bucket and the independent
+ * set over the alive unprotected vertices only. With RLAP_FLAG_FULL_CLIQUE and num_remove >= m_g the result is the
+ * exact Schur complement onto the protected set (a Kron reduction). A non-NULL keep needs a workspace sized with
+ * flags | RLAP_FLAG_KEEP; keep = NULL is rlap_schur_eliminate, bit for bit. keep is read before the call returns. */
+int rlap_schur_eliminate_keep(int64_t n, int64_t nnz, const int32_t* csr_ptr, const int32_t* csr_col, const float* csr_w,
+                              int64_t n_graphs, const int64_t* graph_ptr, const int64_t* num_remove, int o_v, int o_n,
+                              uint64_t seed, int64_t view_base, int64_t n_views, int flags, int64_t pool_cap,
+                              int64_t scratch_cap, void* workspace, size_t workspace_bytes, int64_t* view_rows,
+                              int64_t* stats, const uint8_t* keep, void* stream);
 
 /* ---- emission (replaces the output assembly, preconditioner.cc:435-457 / 789-810 / 916-934) ------
  * Writes the rows of all views back to back, view after view, each view sorted by (col, row):

@@ -15,12 +15,14 @@ FLAG_FULL_CLIQUE = 1
 FLAG_SHARED_ORDER = 2
 FLAG_NO_VALIDATE = 4
 FLAG_CHECK_LIVE = 8
+FLAG_KEEP = 16
 RLAP_ERR_STAR_TOO_LARGE = 6
 
 EXPORTS = [
     "rlap_status_string", "rlap_last_cuda_error", "rlap_version", "rlap_ingest_workspace_bytes", "rlap_ingest",
     "rlap_schur_workspace_bytes", "rlap_schur_eliminate", "rlap_schur_emit", "rlap_approximate_cholesky_host",
     "rlap_free_host", "rlap_schur_colptr", "rlap_expand_cols_host", "rlap_schur_release", "rlap_schur_relabel", "rlap_schur_emit_ids",
+    "rlap_schur_eliminate_keep",
 ]
 
 
@@ -53,6 +55,7 @@ def lib():
     L.rlap_schur_workspace_bytes.argtypes = [i64, i64, i64, i64, i64, i64, ctypes.c_int, ctypes.POINTER(sz)]
     L.rlap_schur_eliminate.argtypes = [i64, i64, P, P, P, i64, P, P, ctypes.c_int, ctypes.c_int, u64, i64, i64,
                                        ctypes.c_int, i64, i64, P, sz, P, P, P]
+    L.rlap_schur_eliminate_keep.argtypes = L.rlap_schur_eliminate.argtypes[:-1] + [P, P]
     L.rlap_schur_emit.argtypes = [i64, i64, P, P, P, i64, P, sz, P, P, P, P, P]
     L.rlap_approximate_cholesky_host.argtypes = [P, i64, i64, i64, ctypes.c_char_p, ctypes.c_char_p, u64,
                                                  ctypes.POINTER(ctypes.POINTER(ctypes.c_double)),

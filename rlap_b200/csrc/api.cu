@@ -19,8 +19,10 @@
 
 namespace rlap {
 cudaError_t launch_hub_index(int n, const int* ptr, int* hubidx, int* count, cudaStream_t stream);
-cudaError_t launch_setup_graphs(int n, int G, const int* gptr, const long long* num_remove, int* gid, int* teff,
-                                cudaStream_t stream);
+cudaError_t launch_setup_graphs(int n, int G, const int* gptr, const long long* num_remove, const int* ucount, int* gid,
+                                int* teff, cudaStream_t stream);
+cudaError_t launch_count_unprotected(int n, const uint8_t* keep, int* flag, int* ucount, long long* blocksum,
+                                     cudaStream_t stream);
 cudaError_t eliminate_grid(int* blocks_out, int o_v, int o_n, int flags);
 cudaError_t launch_eliminate(const SchurParams* groups_host, int K, int blocks, int o_v, int o_n, int flags,
                              cudaStream_t stream);
@@ -265,6 +267,8 @@ struct SchurLayout {
     int* hubidx_dev;           // o_v = random: row of every vertex in the hub head table
     int* hubcount_dev;
     uint64_t* gscratch;        // one scratch slot per block that may own one (NSLOT per group at most)
+    int* unprot_dev;           // keep mask (RLAP_FLAG_KEEP): [n] 1 = unprotected, scanned into ucount_dev [n + 1]
+    int* ucount_dev;
 };
 
 // The views of one call are eliminated by ONE cooperative launch of k_eliminate whose blocks are partitioned into view
@@ -281,7 +285,8 @@ static long long default_scratch_cap(long long n) {
 }
 
 static SchurLayout schur_layout(long long n, long long nnz, long long G, long long V, long long pool_cap,
-                                long long scratch_cap, bool full_clique, void* ws) {
+                                long long scratch_cap, int flags, void* ws) {
+    const bool full_clique = (flags & RLAP_FLAG_FULL_CLIQUE) != 0;
     SchurLayout L;
     memset(&L, 0, sizeof(L));
     if (pool_cap <= 0) pool_cap = default_pool_cap(nnz);
@@ -362,6 +367,10 @@ static SchurLayout schur_layout(long long n, long long nnz, long long G, long lo
         P.hubcount = nullptr;
     }
     P.blocksum = c.take<long long>((size_t)scan_blocks((long long)VN));
+    if (flags & RLAP_FLAG_KEEP) {   // last, so that the pieces above sit where they sit without a mask
+        L.unprot_dev = c.take<int>((size_t)n);
+        L.ucount_dev = c.take<int>((size_t)n + 1);
+    }
     P.gptr = L.gptr_dev;
     P.teff = L.teff_dev;
     P.gid = G > 1 ? L.gid_dev : nullptr;
@@ -384,7 +393,7 @@ int rlap_schur_workspace_bytes(int64_t n, int64_t nnz, int64_t n_graphs, int64_t
     if (!bytes) return RLAP_ERR_INVALID_ARG;
     int st = check_dims(n, nnz, n_graphs, n_views, pool_cap, scratch_cap);
     if (st) return st;
-    *bytes = schur_layout(n, nnz, n_graphs, n_views, pool_cap, scratch_cap, (flags & RLAP_FLAG_FULL_CLIQUE) != 0, nullptr).bytes;
+    *bytes = schur_layout(n, nnz, n_graphs, n_views, pool_cap, scratch_cap, flags, nullptr).bytes;
     return RLAP_OK;
 }
 
@@ -396,12 +405,13 @@ __global__ void k_gather_view_ptr(const long long* outoff, long long n, long lon
     if (v <= V) viewptr[v] = outoff[v * n];
 }
 
-int rlap_schur_eliminate(int64_t n, int64_t nnz, const int32_t* csr_ptr, const int32_t* csr_col, const float* csr_w,
-                         int64_t n_graphs, const int64_t* graph_ptr, const int64_t* num_remove, int o_v, int o_n,
-                         uint64_t seed, int64_t view_base, int64_t n_views, int flags, int64_t pool_cap,
-                         int64_t scratch_cap, void* workspace, size_t workspace_bytes, int64_t* view_rows,
-                         int64_t* stats, void* stream_v) {
+int rlap_schur_eliminate_keep(int64_t n, int64_t nnz, const int32_t* csr_ptr, const int32_t* csr_col, const float* csr_w,
+                              int64_t n_graphs, const int64_t* graph_ptr, const int64_t* num_remove, int o_v, int o_n,
+                              uint64_t seed, int64_t view_base, int64_t n_views, int flags, int64_t pool_cap,
+                              int64_t scratch_cap, void* workspace, size_t workspace_bytes, int64_t* view_rows,
+                              int64_t* stats, const uint8_t* keep, void* stream_v) {
     cudaStream_t stream = (cudaStream_t)stream_v;
+    if (keep) flags |= RLAP_FLAG_KEEP;
     int st = check_dims(n, nnz, n_graphs, n_views, pool_cap, scratch_cap);
     if (st) return st;
     if (!csr_ptr || !graph_ptr || !num_remove || !workspace || !view_rows) return RLAP_ERR_INVALID_ARG;
@@ -410,7 +420,7 @@ int rlap_schur_eliminate(int64_t n, int64_t nnz, const int32_t* csr_ptr, const i
     if (graph_ptr[0] != 0 || graph_ptr[n_graphs] != n) return RLAP_ERR_INVALID_ARG;
     for (int64_t g = 0; g < n_graphs; g++)
         if (graph_ptr[g + 1] < graph_ptr[g]) return RLAP_ERR_INVALID_ARG;
-    SchurLayout L = schur_layout(n, nnz, n_graphs, n_views, pool_cap, scratch_cap, (flags & RLAP_FLAG_FULL_CLIQUE) != 0, workspace);
+    SchurLayout L = schur_layout(n, nnz, n_graphs, n_views, pool_cap, scratch_cap, flags, workspace);
     if (workspace_bytes < L.bytes) return RLAP_ERR_WORKSPACE;
     SchurParams& P = L.P;
     P.ptr = csr_ptr;
@@ -436,8 +446,12 @@ int rlap_schur_eliminate(int64_t n, int64_t nnz, const int32_t* csr_ptr, const i
     }
     CK(cudaMemsetAsync(P.ctr, 0, sizeof(int) * CTR_COUNT, stream));
     CK(cudaMemsetAsync(P.stats, 0, sizeof(unsigned long long) * ST_COUNT, stream));
-    CK(launch_setup_graphs((int)n, (int)n_graphs, L.gptr_dev, L.nrem_dev, n_graphs > 1 ? L.gid_dev : nullptr, L.teff_dev,
-                           stream));
+    if (keep) {
+        CK(launch_count_unprotected((int)n, keep, L.unprot_dev, L.ucount_dev, P.blocksum, stream));
+        P.ucount = L.ucount_dev;
+    }
+    CK(launch_setup_graphs((int)n, (int)n_graphs, L.gptr_dev, L.nrem_dev, P.ucount, n_graphs > 1 ? L.gid_dev : nullptr,
+                           L.teff_dev, stream));
     if (o_v == 0) {
         CK(launch_hub_index((int)n, csr_ptr, L.hubidx_dev, L.hubcount_dev, stream));
         P.hubidx = L.hubidx_dev;
@@ -580,6 +594,16 @@ int rlap_schur_eliminate(int64_t n, int64_t nnz, const int32_t* csr_ptr, const i
     }
     if (hctr[CTR_STATUS] != 0) return hctr[CTR_STATUS];
     return RLAP_OK;
+}
+
+int rlap_schur_eliminate(int64_t n, int64_t nnz, const int32_t* csr_ptr, const int32_t* csr_col, const float* csr_w,
+                         int64_t n_graphs, const int64_t* graph_ptr, const int64_t* num_remove, int o_v, int o_n,
+                         uint64_t seed, int64_t view_base, int64_t n_views, int flags, int64_t pool_cap,
+                         int64_t scratch_cap, void* workspace, size_t workspace_bytes, int64_t* view_rows,
+                         int64_t* stats, void* stream_v) {
+    return rlap_schur_eliminate_keep(n, nnz, csr_ptr, csr_col, csr_w, n_graphs, graph_ptr, num_remove, o_v, o_n, seed,
+                                     view_base, n_views, flags, pool_cap, scratch_cap, workspace, workspace_bytes,
+                                     view_rows, stats, nullptr, stream_v);
 }
 
 static int find_layout(void* workspace, SchurLayout& L) {

@@ -45,7 +45,12 @@ struct ModeParams : SchurParams {
 // list entries, never below 1 once the vertex had an edge (DegreePQDec is a no-op at key 1), 0 for
 // vertices that were isolated from the start; computed inline where it is needed as
 // (state == 4) ? 0 : max(live, 1).
-// state byte: 0 kept (o_v = random, not eligible), 1 pending, 2 eliminated, 4 pending and isolated from the start
+// state byte: 0 kept (o_v = random, not eligible; any order: protected by the keep mask), 1 pending, 2 eliminated,
+// 4 pending and isolated from the start
+// degree / coarsen: a vertex the minimum key, the bucket and the independent-set test see (pending, 1 or 4; not
+// eliminated and not protected). Vertices that are not open may still be appended to a low list (the live-counter
+// crossings of the elimination phase do not read the state byte); the readers of the list drop them.
+__device__ __forceinline__ bool open_st(uint8_t st) { return (st & 5u) != 0; }
 
 // ---------------------------------------------------------------------------------------------
 // star staging
@@ -1345,17 +1350,29 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
         int view = (int)(idx / P.n), v = (int)(idx % P.n);
         *live_p(P, idx) = __ldg(P.ptr + v + 1) - __ldg(P.ptr + v);
         *head_p(P, idx) = -1;
+        // keep mask: protected vertices are state 0; o_v = random ranks c(v), the number of unprotected vertices of
+        // the graph below v, over the graph's m_g unprotected vertices (without a mask c(v) = v - gb and m_g = n_g)
+        const bool prot = P.ucount && __ldg(P.ucount + v + 1) == __ldg(P.ucount + v);
         if (random_order) {
             int g = graph_of(P, v);
             int gb = __ldg(P.gptr + g), ng = __ldg(P.gptr + g + 1) - gb;
-            RankPerm rp;
-            uint32_t oview = (P.flags & 2) ? 0u : (P.view_base + (uint32_t)view);
-            rp.init(P.k0, P.k1, (uint32_t)g, oview, (uint32_t)ng);
-            int rk = (int)rp.rank((uint32_t)(v - gb));
+            int c = v - gb, mg = ng;
+            if (P.ucount) {
+                const int u0 = __ldg(P.ucount + gb);
+                c = __ldg(P.ucount + v) - u0;
+                mg = __ldg(P.ucount + gb + ng) - u0;
+            }
+            int rk = 0x7fffffff;
+            if (!prot) {
+                RankPerm rp;
+                uint32_t oview = (P.flags & 2) ? 0u : (P.view_base + (uint32_t)view);
+                rp.init(P.k0, P.k1, (uint32_t)g, oview, (uint32_t)mg);
+                rk = (int)rp.rank((uint32_t)c);
+            }
             P.rank[idx] = rk;
             P.state[idx] = rk < __ldg(P.teff + g) ? 1 : 0;
         } else {
-            P.state[idx] = (__ldg(P.ptr + v + 1) == __ldg(P.ptr + v)) ? 4 : 1;
+            P.state[idx] = prot ? 0 : (__ldg(P.ptr + v + 1) == __ldg(P.ptr + v)) ? 4 : 1;
             P.candround[idx] = -1;
             P.rank[idx] = -1;   // degree / coarsen: round stamp of the low list
             P.outoff[idx] = 0;  // (round, key) snapshot of phase A (rounds are stored + 1: 0 = never visited)
@@ -1534,7 +1551,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
         lap(ST_T_INIT);
         // degree / coarsen: rounds over the minimum-key bucket of every (view, graph) segment (DESIGN.md §3.4).
         // Full scans of the vertices are only made when a segment's level advances: lvl[seg] is the minimum key
-        // the last full scan found, and every alive vertex whose key is <= lvl[seg] is on the round's low list
+        // the last full scan found, and every open vertex (alive, unprotected) whose key is <= lvl[seg] is on the round's low list
         // (bucket members that were blocked, listed vertices that were not in the bucket, and every vertex whose
         // live counter was seen crossing from above lvl to lvl or below by the elimination phase). While the low
         // list of a segment has an entry in play the bucket is taken from the list alone.
@@ -1575,7 +1592,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
                     if (i < n_in) {
                         const unsigned idx = __ldcg(low_in + i);
                         const uint8_t st = ldcg_u8(P.state + idx);
-                        if (st != 2) {
+                        if (open_st(st)) {
                             seg = (int)(idx / un) * P.G + graph_of(P, (int)(idx % un));
                             key = (st == 4) ? 0 : max(ldcg_i32(live_p(P, idx)), 1);
                             valid = ldcg_i32(P.rem + seg) > 0 && key <= ldcg_i32(P.lvl + seg);
@@ -1672,7 +1689,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
                     }
 #pragma unroll
                     for (int q4 = 0; q4 < 4; q4++) {
-                        const bool valid = nd4[q4] && st4[q4] != 2;
+                        const bool valid = nd4[q4] && open_st(st4[q4]);
                         const int seg = sg4[q4];
                         const int key = valid ? ((st4[q4] == 4) ? 0 : max(lv4[q4], 1)) : INF;
                         if (valid) mark[ix4[q4]] = mark_of(rounds, key);
@@ -1839,7 +1856,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
                 if (i < n_in) {
                     idx = __ldcg(low_in + i);
                     const uint8_t st = ldcg_u8(P.state + idx);
-                    if (st != 2) {
+                    if (open_st(st)) {
                         const int view = (int)(idx / un), v = (int)(idx % un);
                         seg = view * P.G + graph_of(P, v);
                         int m, lv;
@@ -1903,7 +1920,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
                         const unsigned idx = (unsigned)vw4[q4] * un + (unsigned)vx4[q4];
                         const int m = mk4[q4];
                         const int key = (st4[q4] == 4) ? 0 : max(lv4[q4], 1);
-                        const bool alive = m >= 0 && st4[q4] != 2;
+                        const bool alive = m >= 0 && open_st(st4[q4]);
                         const bool member = alive && key == m;
                         const unsigned mm = __ballot_sync(RLAP_FULL_MASK, member);
                         if (member) mbuf[mfill + __popc(mm & lt)] = idx;
@@ -2044,14 +2061,17 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
     }
 }
 
-// gid[v] = graph of vertex v, teff[g] = min(max(num_remove, 0), n_g - 1)
-__global__ void k_setup_graphs(int n, int G, const int* gptr, const long long* num_remove, int* gid, int* teff) {
+// gid[v] = graph of vertex v, teff[g] = min(max(num_remove, 0), n_g - 1); with a keep mask (ucount, see SchurParams)
+// a graph with a protected vertex may lose all its m_g unprotected vertices: teff[g] = min(max(num_remove, 0), m_g)
+__global__ void k_setup_graphs(int n, int G, const int* gptr, const long long* num_remove, const int* ucount, int* gid,
+                               int* teff) {
     long long tid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (tid < G) {
         long long ng = gptr[tid + 1] - gptr[tid];
+        long long mg = ucount ? ucount[gptr[tid + 1]] - ucount[gptr[tid]] : ng;
         long long t = num_remove[tid];
         if (t < 0) t = 0;
-        if (t > ng - 1) t = ng - 1;
+        if (t > (mg < ng ? mg : ng - 1)) t = mg < ng ? mg : ng - 1;
         if (t < 0) t = 0;
         teff[tid] = (int)t;
     }
@@ -2095,13 +2115,27 @@ cudaError_t launch_hub_index(int n, const int* ptr, int* hubidx, int* count, cud
     return cudaGetLastError();
 }
 
-cudaError_t launch_setup_graphs(int n, int G, const int* gptr, const long long* num_remove, int* gid, int* teff,
-                                cudaStream_t stream) {
+cudaError_t launch_setup_graphs(int n, int G, const int* gptr, const long long* num_remove, const int* ucount, int* gid,
+                                int* teff, cudaStream_t stream) {
     long long work = n > G ? n : G;
     int blocks = (int)((work + 255) / 256);
     if (blocks < 1) blocks = 1;
-    k_setup_graphs<<<blocks, 256, 0, stream>>>(n, G, gptr, num_remove, gid, teff);
+    k_setup_graphs<<<blocks, 256, 0, stream>>>(n, G, gptr, num_remove, ucount, gid, teff);
     return cudaGetLastError();
+}
+
+__global__ void k_unprotected(int n, const uint8_t* __restrict__ keep, int* __restrict__ flag) {
+    const int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v < n) flag[v] = keep[v] ? 0 : 1;
+}
+
+// keep mask -> ucount[n + 1]: exclusive prefix count of the unprotected vertices (flag: n ints of scratch)
+cudaError_t launch_count_unprotected(int n, const uint8_t* keep, int* flag, int* ucount, long long* blocksum,
+                                     cudaStream_t stream) {
+    k_unprotected<<<(n + 255) / 256, 256, 0, stream>>>(n, keep, flag);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    return launch_exclusive_scan<int>(flag, n, ucount, blocksum, nullptr, stream);
 }
 
 // One instantiation of k_eliminate per mode. Coarsening fixes the neighbour order (shuffle, preconditioner.cc:831) and

@@ -81,15 +81,17 @@ struct SchurParams {
     const float* w;
     int G;
     const int* gptr;   // [G+1]
-    const int* teff;   // [G] min(num_remove, n_g - 1)
+    const int* teff;   // [G] min(num_remove, n_g - 1), or min(num_remove, m_g) for a graph with a protected vertex
     const int* gid;    // [n] graph of a vertex, or nullptr when G == 1
+    const int* ucount; // keep mask: [n + 1] number of unprotected vertices below v (v is protected iff
+                       // ucount[v + 1] == ucount[v]); nullptr without a mask
     // run
     int o_v, o_n, flags;
     uint32_t k0, k1;
     uint32_t view_base;
     int V;
     // per view state, all indexed [view * n + v]
-    uint8_t* state;    // 0 kept (not eligible), 1 pending, 2 eliminated
+    uint8_t* state;    // 0 kept (not eligible, or protected), 1 pending, 2 eliminated, 4 pending and isolated
     int* lh;           // [V*n][2] interleaved: live = number of raw entries whose neighbour is not eliminated
                        // (RLAP_LIVE_DEAD once the vertex itself is eliminated), head = head of the appended fill-entry
                        // list (pool index, -1 = empty). One 8-byte record: the dead test of a neighbour, the update of

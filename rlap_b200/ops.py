@@ -108,10 +108,31 @@ def prepare(edge_index: Tensor, edge_weights: Optional[Tensor], num_nodes: int,
     return Graph(n, int(nnz.value), ptr, col[: max(int(nnz.value), 1)], cw[: max(int(nnz.value), 1)], gp, dev)
 
 
+def _keep_mask(keep, n: int, device) -> Tensor:
+    """keep as a device uint8 [n] of 0 / 1; ValueError for a mask of another length, shape or dtype (a bool or integer
+    mask with values other than 0 and 1 included)"""
+    if isinstance(keep, Tensor):
+        k = keep.detach()
+    else:
+        a = np.asarray(keep)
+        if a.dtype.kind not in "biu":
+            raise ValueError(f"keep must be a bool or 0/1 mask, got dtype {a.dtype}")
+        k = torch.from_numpy(np.ascontiguousarray(a))
+    if k.dtype != torch.bool and (k.is_floating_point() or k.is_complex()):
+        raise ValueError(f"keep must be a bool or 0/1 mask, got dtype {k.dtype}")
+    if k.dim() != 1 or k.shape[0] != n:
+        raise ValueError(f"keep must have one entry per node ({n}), got shape {tuple(k.shape)}")
+    k = k.to(device=device)
+    if k.dtype != torch.bool:
+        if n > 0 and bool(((k != 0) & (k != 1)).any()):
+            raise ValueError("keep must be a bool or 0/1 mask")
+    return k.to(torch.uint8).contiguous()
+
+
 def schur_views(graph: Graph, num_remove, o_v: str, o_n: str, num_views: int = 1, seed: Optional[int] = None,
                 view_base: int = 0, full_clique: bool = False, shared_order: bool = False, dtype=torch.float64,
                 pool_cap: int = 0, scratch_cap: int = 0, return_stats: bool = False, colptr: bool = False,
-                check_live: bool = False, weights: bool = True, relabel: bool = False):
+                check_live: bool = False, weights: bool = True, relabel: bool = False, keep=None):
     """num_views independent randomized Schur-complement views of `graph`.
 
     Returns (edge_info, view_ptr): edge_info is [sum E'_v, 3] (row, col, weight) of `dtype`
@@ -125,7 +146,11 @@ def schur_views(graph: Graph, num_remove, o_v: str, o_n: str, num_views: int = 1
     relabel=True: survivor compaction + relabelling inside the emission (what the reference's adapters do afterwards
     with torch.unique + subgraph(relabel_nodes=True), scripts/augmentor_benchmarks.py:149-155): the row / col ids of
     view v are ranks among that view's vertices with at least one edge, and the call returns one more value, `newid`
-    int32 [num_views, n] (-1 for vertices without edges; `(newid[v] >= 0).nonzero()` is the sorted node list)."""
+    int32 [num_views, n] (-1 for vertices without edges; `(newid[v] >= 0).nonzero()` is the sorted node list).
+    keep: a bool or 0/1 mask of length n (tensor on any device, array or sequence), or None. A marked vertex is
+    protected: no view eliminates it, and a graph with a protected vertex may lose every other vertex (num_remove is
+    capped at its number of unprotected vertices instead of n_g - 1). With full_clique=True and num_remove >= that
+    number the views are the exact Schur complement onto the protected set (a Kron reduction)."""
     assert o_v in _O_V
     assert o_n in _O_N
     L = _native.lib()
@@ -138,6 +163,9 @@ def schur_views(graph: Graph, num_remove, o_v: str, o_n: str, num_views: int = 1
     flags |= _native.FLAG_CHECK_LIVE if check_live else 0
     flags |= _DEBUG_FLAGS
     V = int(num_views)
+    kmask = None if keep is None else _keep_mask(keep, graph.n, dev)
+    if kmask is not None:
+        flags |= _native.FLAG_KEEP
     if full_clique:  # test mode: cliques instead of trees, multi-edges pile up until a vertex goes
         pool_cap = pool_cap or 8 * graph.nnz + 4096
         scratch_cap = scratch_cap or (1 << 18)
@@ -150,11 +178,14 @@ def schur_views(graph: Graph, num_remove, o_v: str, o_n: str, num_views: int = 1
             ws = torch.empty(wsb.value, dtype=torch.uint8, device=dev)
             rows = np.zeros(V, dtype=np.int64)
             stats = np.zeros(16, dtype=np.int64)
-            st = L.rlap_schur_eliminate(graph.n, graph.nnz, graph.ptr.data_ptr(), graph.col.data_ptr(),
-                                        graph.w.data_ptr(), G, graph.graph_ptr.ctypes.data, nr.ctypes.data,
-                                        _native.OV[o_v], _native.ON[o_n], seed & 0xFFFFFFFFFFFFFFFF, view_base, V, flags,
-                                        pool_cap, scratch_cap, ws.data_ptr(), wsb.value, rows.ctypes.data, stats.ctypes.data,
-                                        stream)
+            args = (graph.n, graph.nnz, graph.ptr.data_ptr(), graph.col.data_ptr(), graph.w.data_ptr(), G,
+                    graph.graph_ptr.ctypes.data, nr.ctypes.data, _native.OV[o_v], _native.ON[o_n],
+                    seed & 0xFFFFFFFFFFFFFFFF, view_base, V, flags, pool_cap, scratch_cap, ws.data_ptr(), wsb.value,
+                    rows.ctypes.data, stats.ctypes.data)
+            if kmask is None:
+                st = L.rlap_schur_eliminate(*args, stream)
+            else:
+                st = L.rlap_schur_eliminate_keep(*args, kmask.data_ptr(), stream)
             if st == _native.RLAP_ERR_POOL_OVERFLOW:
                 pool_cap = 2 * int(stats[6])
                 del ws
@@ -224,11 +255,12 @@ def expand_cols(colptr_host: Tensor, view_ptr: Tensor, out: Optional[Tensor] = N
 
 def approximate_cholesky_batched(edge_index: Tensor, edge_weights: Optional[Tensor], num_nodes: int, num_remove,
                                  o_v: str, o_n: str, num_views: int = 1, graph_ptr=None, seed: Optional[int] = None,
-                                 dtype=torch.float64, **kw) -> Tuple[Tensor, Tensor]:
+                                 dtype=torch.float64, keep=None, **kw) -> Tuple[Tensor, Tensor]:
     """Batched variant: `num_views` views of one graph, or of every graph of a batch (graph_ptr),
-    in one call. Returns (edge_info [sum E', 3], view_ptr [num_views + 1])."""
+    in one call. Returns (edge_info [sum E', 3], view_ptr [num_views + 1]). keep: protected vertices, as in
+    schur_views."""
     g = prepare(edge_index, edge_weights, num_nodes, graph_ptr=graph_ptr)
-    out, vp = schur_views(g, num_remove, o_v, o_n, num_views=num_views, seed=seed, dtype=dtype, **kw)
+    out, vp = schur_views(g, num_remove, o_v, o_n, num_views=num_views, seed=seed, dtype=dtype, keep=keep, **kw)
     if not edge_index.is_cuda and dtype is not None:
         out = out.to(edge_index.device)
     return out, vp
@@ -242,6 +274,7 @@ def approximate_cholesky(
     o_v: str,
     o_n: str,
     seed: Optional[int] = None,
+    keep=None,
 ) -> Tensor:
     """
     Compute the randomized Schur complement of the graph Laplacian (same contract as the
@@ -252,10 +285,12 @@ def approximate_cholesky(
     edge_index : Tensor [2, E] of node ids (both directions of every edge present).
     edge_weights : Tensor [E] or [1, E] of edge weights, or None for unit weights.
     num_nodes : total number of nodes.
-    num_remove : number of nodes to eliminate (capped at num_nodes - 1).
+    num_remove : number of nodes to eliminate (capped at num_nodes - 1, or at the number of unprotected nodes when
+        keep marks at least one node).
     o_v : elimination order, one of ["random", "degree", "coarsen"].
     o_n : neighbour order, one of ["asc", "desc", "random"].
     seed : optional 64-bit seed (extension; the reference is unseedable).
+    keep : optional bool or 0/1 mask of length num_nodes (extension): marked nodes are never eliminated.
 
     Returns:
     --------
@@ -266,7 +301,7 @@ def approximate_cholesky(
     assert o_v in _O_V
     assert o_n in _O_N
     g = prepare(edge_index, edge_weights, num_nodes)
-    out, _ = schur_views(g, int(num_remove), o_v, o_n, num_views=1, seed=seed, dtype=torch.float64)
+    out, _ = schur_views(g, int(num_remove), o_v, o_n, num_views=1, seed=seed, dtype=torch.float64, keep=keep)
     return out.to(edge_index.device)
 
 
