@@ -9,7 +9,8 @@ import subprocess
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_LIB_PATH = os.environ.get("RLAP_ORACLE_LIB") or os.path.join(_HERE, "_build", "liboracle.so")   # override: experiments with an older build
+_OVERRIDE = os.environ.get("RLAP_ORACLE_LIB")   # experiments with an older build: loaded as it is, never built
+_LIB_PATH = _OVERRIDE or os.path.join(_HERE, "_build", "liboracle.so")
 _lib = None
 
 OV = {"random": 0, "degree": 1, "coarsen": 2}
@@ -25,8 +26,8 @@ def build():
 def lib():
     global _lib
     if _lib is None:
-        if not os.path.exists(_LIB_PATH):
-            build()
+        if not _OVERRIDE:
+            build()   # a no-op when the library is newer than rlap_oracle.cc; a stale one is rebuilt, never loaded
         L = ctypes.CDLL(_LIB_PATH)
         P = ctypes.c_void_p
         L.oracle_ref_approximate_cholesky.argtypes = [
@@ -40,7 +41,7 @@ def lib():
         L.oracle_ingest.restype = ctypes.c_int64
         L.oracle_keyed_schur.argtypes = [
             ctypes.c_int64, P, P, P, ctypes.c_int64, P, P, ctypes.c_int, ctypes.c_int, ctypes.c_uint64,
-            ctypes.c_uint32, ctypes.c_int, P, P, P, ctypes.c_int64, P, P]
+            ctypes.c_uint32, ctypes.c_int, P, P, P, ctypes.c_int64, P, P, P]
         L.oracle_keyed_schur.restype = ctypes.c_int64
         L.oracle_ref_random_order.argtypes = [ctypes.c_int64, ctypes.c_uint64, P]
         L.oracle_rank_perm.argtypes = [ctypes.c_uint64, ctypes.c_uint32, ctypes.c_uint32, ctypes.c_uint32, P]
@@ -113,9 +114,15 @@ def ingest(edge_index, weights, n):
 
 
 def keyed_schur(ptr, col, w, num_remove, o_v, o_n, seed=0, view=0, graph_ptr=None, flags=0, return_stats=False,
-                return_order=False):
-    """keyed mode on a coalesced CSR: returns (row, col, w) sorted by (col,row)."""
+                return_order=False, keep=None):
+    """keyed mode on a coalesced CSR: returns (row, col, w) sorted by (col,row), then the stats and the elimination
+    order if asked for. keep (n entries, nonzero = protected; None = no mask): DESIGN.md §3.7."""
     n = ptr.shape[0] - 1
+    if keep is not None:
+        keep = np.asarray(keep)
+        if keep.shape != (n,):
+            raise ValueError(f"keep must have one entry per vertex ({n}), got shape {keep.shape}")
+        keep = np.ascontiguousarray(keep != 0, dtype=np.uint8)
     if graph_ptr is None:
         graph_ptr = np.array([0, n], dtype=np.int64)
     graph_ptr = np.ascontiguousarray(graph_ptr, dtype=np.int64)
@@ -133,7 +140,8 @@ def keyed_schur(ptr, col, w, num_remove, o_v, o_n, seed=0, view=0, graph_ptr=Non
         ow = np.zeros(cap, dtype=np.float32)
         rows = lib().oracle_keyed_schur(n, ptr.ctypes.data, col.ctypes.data, w.ctypes.data, G, graph_ptr.ctypes.data,
                                         t.ctypes.data, OV[o_v], ON[o_n], seed, view, flags, orow.ctypes.data,
-                                        ocol.ctypes.data, ow.ctypes.data, cap, stats.ctypes.data, order.ctypes.data)
+                                        ocol.ctypes.data, ow.ctypes.data, cap, stats.ctypes.data, order.ctypes.data,
+                                        None if keep is None else keep.ctypes.data)
         if rows <= cap:
             break
         cap = rows

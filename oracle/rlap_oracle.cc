@@ -22,7 +22,9 @@
 //      (rows, columns AND fp32 weights). It shares the sampling rule (A.2: neighbour j gets one
 //      fill edge to a later neighbour k drawn with probability proportional to weight, weight
 //      w_j (S - C_j) / S), the coarsening rule (A.4) and the emission rule (A.5) with mode (1).
-//      Statistical equivalence of (1) and (2) is tested in tests/test_oracle_stats.py.
+//      Statistical equivalence of (1) and (2) is tested in tests/test_oracle_keyed.py. An optional keep mask
+//      (DESIGN.md §3.7) protects vertices from elimination; without one the driver is the unmasked specification.
+//      Its bits are pinned by stored digests (tests/test_oracle_keyed_pin.py).
 //
 // Build: make -C oracle oracle   (g++ -O3 -std=c++17 -shared -fPIC)
 #include <algorithm>
@@ -574,10 +576,6 @@ static void order_star(Star& s, int o_n) {
 }
 
 struct Stats { int64_t D = 0, F = 0, maxlen = 0, rounds = 0, Draw = 0; };
-// optional histograms of the raw / merged star sizes (oracle_set_hist): [0..63] exact, [64] = 64 and above
-static int64_t* g_hist_raw = nullptr;
-static int64_t* g_hist_len = nullptr;
-static int64_t* g_emit_counts = nullptr;   // optional [4]: survivors with entries, with a multi-edge, raw entries, merged rows
 
 static void add_edge(Graph& g, int32_t a, int32_t b, float w) {
     g.adj[(size_t)a].push_back(Entry{b, w});
@@ -593,8 +591,6 @@ static void eliminate(Graph& g, int32_t i, int o_v, int o_n, int flags, const Ph
     st.D += s.lraw;
     int64_t L = (int64_t)s.m.size();
     st.maxlen = std::max(st.maxlen, L);
-    if (g_hist_raw) g_hist_raw[std::min<int64_t>(s.lraw, 64)]++;
-    if (g_hist_len) g_hist_len[std::min<int64_t>(L, 64)]++;
     for (Merged& mm : s.m) {
         uint32_t o[4];
         ph((uint32_t)i, (uint32_t)mm.nbr, view, TAG_STAR, o);
@@ -727,11 +723,17 @@ int64_t oracle_ingest(const int64_t* src, const int64_t* dst, const float* w, in
 // Output rows sorted by (col, row); returns E'. out_* must hold >= nnz entries (E' <= nnz + 0: live
 // multigraph entries never exceed the input's, see DESIGN.md §3.6).
 // stats: D, F, maxlen, rounds, Draw. order_out (optional, n entries): elimination round of each vertex, -1 if kept.
+// keep (optional, n entries; NULL = no mask, DESIGN.md §3.7): a nonzero flag protects the vertex, it is never
+// eliminated. For graph g with m_g unprotected vertices: t_g = min(max(num_remove, 0), m_g) if g has a protected vertex,
+// else min(max(num_remove, 0), n_g - 1). o_v = random ranks the unprotected vertices, numbered by ascending id, with the
+// keyed permutation over m_g; degree / coarsen take the minimum key, the bucket and the independent-set test over the
+// alive unprotected vertices only.
 int64_t oracle_keyed_schur(int64_t n, const int64_t* ptr, const int32_t* col, const float* w, int64_t G,
                            const int64_t* graph_ptr, const int64_t* num_remove, int o_v, int o_n, uint64_t seed,
                            uint32_t view, int flags, int32_t* out_row, int32_t* out_col, float* out_w,
-                           int64_t out_cap, int64_t* stats, int32_t* order_out) {
+                           int64_t out_cap, int64_t* stats, int32_t* order_out, const uint8_t* keep) {
     using namespace keyed;
+    auto prot = [&](int64_t v) { return keep && keep[v] != 0; };
     Graph g;
     g.n = n;
     g.adj.resize((size_t)n);
@@ -747,31 +749,38 @@ int64_t oracle_keyed_schur(int64_t n, const int64_t* ptr, const int32_t* col, co
     if (order_out) for (int64_t v = 0; v < n; v++) order_out[v] = -1;
     for (int64_t gi = 0; gi < G; gi++) {
         int64_t b = graph_ptr[gi], e = graph_ptr[gi + 1], ng = e - b;
-        int64_t t = std::min<int64_t>(std::max<int64_t>(num_remove[gi], 0), std::max<int64_t>(ng - 1, 0));
+        // the unprotected vertices of the graph, ascending: c(v) = position in this list
+        std::vector<int32_t> unprot;
+        for (int64_t v = b; v < e; v++)
+            if (!prot(v)) unprot.push_back((int32_t)v);
+        const int64_t mg = (int64_t)unprot.size();
+        // without a protected vertex one vertex always survives (the reference's cap); with one, every other may go
+        int64_t t = std::min<int64_t>(std::max<int64_t>(num_remove[gi], 0), mg < ng ? mg : std::max<int64_t>(ng - 1, 0));
         if (o_v == OV_RANDOM) {
             // the t vertices of lowest rank go, in rank order: strictly sequential here; the CUDA path
             // runs any schedule that respects "lower-ranked adjacent vertex first" (SURVEY.md App. B.4)
-            RankPerm rp(ph, (uint32_t)gi, (flags & FLAG_SHARED_ORDER) ? 0u : view, (uint32_t)ng);
-            std::vector<int32_t> by_rank((size_t)ng);
-            for (int64_t v = b; v < e; v++) by_rank[(size_t)rp.rank((uint32_t)(v - b))] = (int32_t)v;
+            RankPerm rp(ph, (uint32_t)gi, (flags & FLAG_SHARED_ORDER) ? 0u : view, (uint32_t)mg);
+            std::vector<int32_t> by_rank((size_t)mg);
+            for (int64_t c = 0; c < mg; c++) by_rank[(size_t)rp.rank((uint32_t)c)] = unprot[(size_t)c];
             for (int64_t k = 0; k < t; k++) {
                 eliminate(g, by_rank[(size_t)k], o_v, o_n, flags, ph, view, st);
                 if (order_out) order_out[by_rank[(size_t)k]] = (int32_t)k;
             }
             st.rounds = std::max(st.rounds, t);
         } else {
-            // degree / coarsen: rounds over the minimum-key bucket (DESIGN.md §3.4)
+            // degree / coarsen: rounds over the minimum-key bucket of the alive unprotected vertices (DESIGN.md §3.4)
+            auto open = [&](int64_t v) { return !g.elim[(size_t)v] && !prot(v); };
             int64_t rem = t, round = 0;
             while (rem > 0) {
                 int32_t m = 0x7fffffff;
                 for (int64_t v = b; v < e; v++)
-                    if (!g.elim[(size_t)v]) m = std::min(m, key_of(g, (int32_t)v));
+                    if (open(v)) m = std::min(m, key_of(g, (int32_t)v));
                 std::vector<int32_t> I;
                 for (int64_t v = e - 1; v >= b; v--) {   // descending id = ascending tie-break
-                    if (g.elim[(size_t)v] || key_of(g, (int32_t)v) != m) continue;
+                    if (!open(v) || key_of(g, (int32_t)v) != m) continue;
                     bool ok = true;
                     for (const Entry& en : g.adj[(size_t)v])
-                        if (!g.elim[(size_t)en.nbr] && en.nbr > v && key_of(g, en.nbr) == m) { ok = false; break; }
+                        if (open(en.nbr) && en.nbr > v && key_of(g, en.nbr) == m) { ok = false; break; }
                     if (ok) I.push_back((int32_t)v);
                 }
                 if ((int64_t)I.size() > rem) I.resize((size_t)rem);  // keep the highest ids
@@ -791,12 +800,6 @@ int64_t oracle_keyed_schur(int64_t n, const int64_t* ptr, const int32_t* col, co
     for (int64_t v = 0; v < n; v++) {
         if (g.elim[(size_t)v]) continue;
         gather_star(g, (int32_t)v, s);
-        if (keyed::g_emit_counts && s.lraw > 0) {
-            keyed::g_emit_counts[0]++;
-            if ((int64_t)s.m.size() != s.lraw) keyed::g_emit_counts[1]++;
-            keyed::g_emit_counts[2] += s.lraw;
-            keyed::g_emit_counts[3] += (int64_t)s.m.size();
-        }
         for (const Merged& mm : s.m) {
             if (rows < out_cap) { out_row[rows] = mm.nbr; out_col[rows] = (int32_t)v; out_w[rows] = mm.wf; }
             rows++;
@@ -807,10 +810,6 @@ int64_t oracle_keyed_schur(int64_t n, const int64_t* ptr, const int32_t* col, co
 }
 
 }  // extern "C"
-
-// histograms of the star sizes seen by the keyed eliminations that follow (65 bins each; nullptr switches them off)
-extern "C" void oracle_set_hist(int64_t* raw, int64_t* len) { keyed::g_hist_raw = raw; keyed::g_hist_len = len; }
-extern "C" void oracle_set_emit_counts(int64_t* c) { keyed::g_emit_counts = c; }
 
 extern "C" void oracle_rank_perm(uint64_t seed, uint32_t graph, uint32_t view, uint32_t n_g, uint32_t* out) {
     keyed::Philox ph{(uint32_t)seed, (uint32_t)(seed >> 32)};

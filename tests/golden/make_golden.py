@@ -13,7 +13,13 @@ writes tests/golden/ref_build/cases.npz instead: the inputs of the reference-bui
 (tests/util.py reference_build_cases, seeds REF_BUILD_SEEDS) and, per (case, o_v, o_n), the row count, the SHA-256
 of the whole [E',3] float64 output and a seeded sample of its rows. Whole outputs of these larger graphs would be
 ~1.3 MB. The outputs come from the reference build, or with --from-oracle-ref-mode from the oracle's reference
-mode; the file's `source` entry says which."""
+mode; the file's `source` entry says which.
+
+    python tests/golden/make_golden.py --keyed-cases
+
+writes tests/golden/keyed/cases.npz: for every run of tests/util.py keyed_pin_runs, its id and the SHA-256 of the
+keyed oracle's output (row, col and fp32 weight bytes), stats and elimination order (util.keyed_digest). Regenerating
+on a later tree must give the same arrays; `source` records the commit the digests were first taken on."""
 import os
 import sys
 
@@ -27,6 +33,7 @@ from tests import util  # noqa: E402
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 REF_BUILD_PATH = os.path.join(HERE, "ref_build", "cases.npz")
+KEYED_PATH = os.path.join(HERE, "keyed", "cases.npz")
 SAMPLE_ROWS = 64
 
 # what --from-oracle-ref-mode records as the source: refmode in oracle/rlap_oracle.cc, ref_driver.cc and
@@ -34,6 +41,9 @@ SAMPLE_ROWS = 64
 # mode bit for bit with the reference build on exactly these inputs and seeds
 ORACLE_SOURCE = ("oracle reference mode (oracle/rlap_oracle.cc refmode, unchanged since c4ca53b, where it matched the "
                  "reference build bit for bit on these cases)")
+
+KEYED_SOURCE = ("oracle keyed mode at commit 8ecb4b5 (unmasked runs: oracle_keyed_schur; masked runs: the keep-mask "
+                "copy of its driver that commit had)")
 
 
 def sample_index(rows: int) -> np.ndarray:
@@ -86,8 +96,21 @@ def ref_build_cases(from_oracle: bool):
     print("reference-build cases written to", REF_BUILD_PATH, "from", source)
 
 
+def keyed_cases():
+    from oracle import port
+    ids, digest = [], []
+    for case, ptr, col, w, kw in util.keyed_pin_runs(port):
+        ids.append(case)
+        digest.append(util.keyed_digest(port, ptr, col, w, kw))
+    os.makedirs(os.path.dirname(KEYED_PATH), exist_ok=True)
+    np.savez_compressed(KEYED_PATH, source=np.array(KEYED_SOURCE), case=np.array(ids), digest=np.stack(digest))
+    print(len(ids), "keyed-mode digests written to", KEYED_PATH)
+
+
 if __name__ == "__main__":
     if "--ref-build-cases" in sys.argv:
         ref_build_cases("--from-oracle-ref-mode" in sys.argv)
+    elif "--keyed-cases" in sys.argv:
+        keyed_cases()
     else:
         main()

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 import torch
 
-from tests import keep_oracle, util
+from tests import util
 
 pytestmark = pytest.mark.gpu
 
@@ -27,12 +27,7 @@ def _mask_cases():
     cases.append(("ba300", ei, n, None, [150, n], masks))
     ei, gp = graphs.proteins_like_batch(40, seed=3)
     n = int(gp[-1])
-    whole = np.zeros(n, dtype=bool)
-    whole[gp[3]:gp[4]] = True                                   # one whole graph of the batch
-    single = np.ones(n, dtype=bool)
-    for g in range(gp.shape[0] - 1):                            # a single unprotected vertex per graph
-        single[gp[g] + g % (gp[g + 1] - gp[g])] = False
-    masks = [("rand50", rng.random(n) < 0.5), ("whole_graph", whole), ("single_free", single)]
+    masks = [("rand50", rng.random(n) < 0.5)] + util.batch_masks(gp)
     cases.append(("proteins40", ei, n, gp, [np.diff(gp) // 2, np.diff(gp)], masks))
     return cases
 
@@ -40,7 +35,7 @@ def _mask_cases():
 def _check_views(oracle_port, optr, ocol, ow, row, col, wt, vp, t, o_v, o_n, seed, view_base, gptr, keep, flags=0,
                  what=""):
     for v in range(vp.shape[0] - 1):
-        r0, c0, w0 = keep_oracle.keyed_schur(optr, ocol, ow, t, o_v, o_n, seed=seed, view=view_base + v,
+        r0, c0, w0 = oracle_port.keyed_schur(optr, ocol, ow, t, o_v, o_n, seed=seed, view=view_base + v,
                                              graph_ptr=gptr, flags=flags, keep=keep)
         s, e = vp[v], vp[v + 1]
         assert e - s == r0.shape[0], (what, v, e - s, r0.shape[0])
@@ -146,7 +141,7 @@ def test_arxiv_shape_half_protected_matches_oracle(oracle_port, o_v):
     g = rlap_b200.prepare(torch.from_numpy(ei).cuda(), None, n)
     (row, col, wt), vp = rlap_b200.schur_views(g, n, o_v, "asc", num_views=1, seed=13, dtype=None, keep=keep)
     row, col, wt = row.cpu().numpy(), col.cpu().numpy(), wt.cpu().numpy()
-    r0, c0, w0 = keep_oracle.keyed_schur(optr, ocol, ow, n, o_v, "asc", seed=13, keep=keep)
+    r0, c0, w0 = oracle_port.keyed_schur(optr, ocol, ow, n, o_v, "asc", seed=13, keep=keep)
     assert np.array_equal(row, r0) and np.array_equal(col, c0)
     assert np.array_equal(wt.view(np.uint32), w0.view(np.uint32))
     assert keep[row].all() and keep[col].all()                  # only protected vertices are left

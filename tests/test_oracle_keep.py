@@ -1,12 +1,11 @@
 """The keyed specification with a keep mask (DESIGN.md §3.7): protected vertices are never eliminated. The sequential
-form is tests/native/keep_oracle.cc, the keyed oracle's driver restated with the mask. An all-false mask (and no mask)
-gives the oracle's own output; the invariants, the cap, the degree bucket over unprotected vertices and the exact Kron
-reduction of full-clique mode."""
+form is the keyed oracle's `keep` argument. An all-false mask (and no mask) gives the oracle's unmasked output; the
+invariants, the cap, the degree bucket over unprotected vertices and the exact Kron reduction of full-clique mode."""
 import numpy as np
 import pytest
 
 from rlap_b200 import graphs
-from tests import keep_oracle, util
+from tests import util
 
 
 def _t_eff(num_remove, n_g, m_g):
@@ -15,15 +14,15 @@ def _t_eff(num_remove, n_g, m_g):
 
 @pytest.mark.parametrize("case", util.small_cases(), ids=lambda c: c[0])
 def test_all_false_mask_is_no_mask(oracle_port, case):
-    """no mask and an all-false mask both give the keyed oracle's own output, bit for bit, with the same stats and
-    elimination order"""
+    """keep=None and an all-false mask both give the keyed oracle's unmasked output, bit for bit, with the same stats
+    and elimination order"""
     name, ei, n, gp, t = case
     ptr, col, w = oracle_port.ingest(ei, None, n)
     for o_v, o_n in util.COMBOS:
         a = oracle_port.keyed_schur(ptr, col, w, t, o_v, o_n, seed=5, graph_ptr=gp, return_stats=True,
                                     return_order=True)
         for keep in (None, np.zeros(n, dtype=bool)):
-            b = keep_oracle.keyed_schur(ptr, col, w, t, o_v, o_n, seed=5, graph_ptr=gp, return_stats=True,
+            b = oracle_port.keyed_schur(ptr, col, w, t, o_v, o_n, seed=5, graph_ptr=gp, return_stats=True,
                                         return_order=True, keep=keep)
             for x, y in zip(a[:3], b[:3]):
                 assert np.array_equal(x.view(np.uint32), y.view(np.uint32)), (name, o_v, o_n)
@@ -31,7 +30,7 @@ def test_all_false_mask_is_no_mask(oracle_port, case):
 
 
 def _check_invariants(oracle_port, ptr, col, w, n, gp, t, o_v, o_n, keep, seed):
-    r, c, wt, order = keep_oracle.keyed_schur(ptr, col, w, t, o_v, o_n, seed=seed, graph_ptr=gp, return_order=True,
+    r, c, wt, order = oracle_port.keyed_schur(ptr, col, w, t, o_v, o_n, seed=seed, graph_ptr=gp, return_order=True,
                                               keep=keep)
     gp = np.array([0, n]) if gp is None else gp
     tt = np.broadcast_to(np.asarray(t), (gp.shape[0] - 1,))
@@ -79,12 +78,12 @@ def test_fully_protected_graph_returns_its_input(oracle_port, o_v):
     w = util.sym_weights(ei)
     ptr, col, ww = oracle_port.ingest(ei, w, n)
     owner = np.repeat(np.arange(n), np.diff(ptr))
-    r, c, wt = keep_oracle.keyed_schur(ptr, col, ww, n, o_v, "asc", seed=1, keep=np.ones(n, dtype=bool))
+    r, c, wt = oracle_port.keyed_schur(ptr, col, ww, n, o_v, "asc", seed=1, keep=np.ones(n, dtype=bool))
     assert np.array_equal(r, col) and np.array_equal(c, owner) and np.array_equal(wt, ww)
     # one whole graph of a batch protected, the others reduced to one vertex: that graph's rows are its input
     keep = np.zeros(n, dtype=bool)
     keep[gp[4]:gp[5]] = True
-    r, c, wt = keep_oracle.keyed_schur(ptr, col, ww, n, o_v, "asc", seed=1, graph_ptr=gp, keep=keep)
+    r, c, wt = oracle_port.keyed_schur(ptr, col, ww, n, o_v, "asc", seed=1, graph_ptr=gp, keep=keep)
     sel = (owner >= gp[4]) & (owner < gp[5])
     mine = (c >= gp[4]) & (c < gp[5])
     assert np.array_equal(r[mine], col[sel]) and np.array_equal(c[mine], owner[sel]) and np.array_equal(wt[mine], ww[sel])
@@ -115,7 +114,7 @@ def test_full_clique_is_kron_reduction(oracle_port, case, o_v):
     rng = np.random.default_rng(3)
     masks = [rng.random(n) < f for f in (0.1, 0.3, 0.7)] + [np.arange(n) % 17 == 0]
     for keep in masks:
-        r, c, wt = keep_oracle.keyed_schur(ptr, col, ww, n, o_v, "asc", seed=7, flags=oracle_port.FLAG_FULL_CLIQUE,
+        r, c, wt = oracle_port.keyed_schur(ptr, col, ww, n, o_v, "asc", seed=7, flags=oracle_port.FLAG_FULL_CLIQUE,
                                            keep=keep)
         k = np.where(keep)[0]
         Ls = util.laplacian(r, c, wt, n)[np.ix_(k, k)]
@@ -136,7 +135,7 @@ def test_degree_bucket_ignores_protected_vertices(oracle_port, o_v):
         free = np.where(~keep)[0]
         m = deg[free].min()
         want = free[deg[free] == m][-1]                        # highest id among the unprotected of minimum degree
-        _, _, _, order = keep_oracle.keyed_schur(ptr, col, w, 1, o_v, "asc", seed=trial, keep=keep, return_order=True)
+        _, _, _, order = oracle_port.keyed_schur(ptr, col, w, 1, o_v, "asc", seed=trial, keep=keep, return_order=True)
         assert np.where(order >= 0)[0].tolist() == [want]
 
 
@@ -149,7 +148,7 @@ def test_random_order_ranks_the_unprotected_vertices(oracle_port):
     keep = np.random.default_rng(2).random(n) < 0.5
     free = np.where(~keep)[0]
     for view in (0, 3):
-        _, _, _, order = keep_oracle.keyed_schur(ptr, col, w, t, "random", "asc", seed=11, view=view, keep=keep,
+        _, _, _, order = oracle_port.keyed_schur(ptr, col, w, t, "random", "asc", seed=11, view=view, keep=keep,
                                                  return_order=True)
         rank = oracle_port.rank_perm(11, 0, view, free.shape[0])
         by_rank = free[np.argsort(rank)]
