@@ -82,7 +82,9 @@ int rlap_ingest(const int64_t* src, const int64_t* dst, const float* w, int64_t 
  * getSchurComplement, preconditioner.cc:348-476, 713-825, 835-957) --------------------------------
  * Produces n_views independent views (view ids view_base .. view_base+n_views-1; randomness is a
  * pure function of (seed, view id, vertex, neighbour), so results do not depend on how views are
- * sharded over GPUs). graph_ptr: HOST int64[n_graphs+1]; num_remove: HOST int64[n_graphs].
+ * sharded over GPUs). The limits of one call: view ids are 32-bit (view_base + n_views <= 2^32,
+ * RLAP_ERR_INVALID_ARG otherwise) and n_views * n < 2^30 (work-list positions are 32-bit).
+ * graph_ptr: HOST int64[n_graphs+1]; num_remove: HOST int64[n_graphs].
  * pool_cap: fill-edge pool entries per view (0 = default 2*nnz + 4096). scratch_cap: largest star
  * (raw live entries) the global scratch path accepts (0 = default min(n, 65536); rounded up to a power of two, the
  * size a star is padded to when it is sorted; a larger star returns

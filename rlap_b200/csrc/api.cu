@@ -417,6 +417,8 @@ int rlap_schur_eliminate_keep(int64_t n, int64_t nnz, const int32_t* csr_ptr, co
     if (!csr_ptr || !graph_ptr || !num_remove || !workspace || !view_rows) return RLAP_ERR_INVALID_ARG;
     if (nnz > 0 && (!csr_col || !csr_w)) return RLAP_ERR_INVALID_ARG;
     if (o_v < 0 || o_v > 2 || o_n < 0 || o_n > 2 || view_base < 0) return RLAP_ERR_INVALID_ARG;
+    // view ids are 32-bit words of the Philox counter: a larger id would wrap onto view (id mod 2^32)
+    if (view_base > (1LL << 32) - n_views) return RLAP_ERR_INVALID_ARG;
     if (graph_ptr[0] != 0 || graph_ptr[n_graphs] != n) return RLAP_ERR_INVALID_ARG;
     for (int64_t g = 0; g < n_graphs; g++)
         if (graph_ptr[g + 1] < graph_ptr[g]) return RLAP_ERR_INVALID_ARG;

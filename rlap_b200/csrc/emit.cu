@@ -81,30 +81,32 @@ __global__ void __launch_bounds__(256) k_emit_base(SchurParams P) {
     }
 }
 
-// Fill entries: grid-stride over the view's pool (blockIdx.y = view), one thread per fill edge = the two entries
-// (j <- k), (k <- j) it left in adjacent slots (reservations are even, so pairs never straddle); if both endpoints
-// are alive each entry goes to the tail of its owner's staging segment, filled from the end backwards (the front is
-// where the alive base entries of a merge-path vertex go; cursor[v] counts the fills of v)
+// Fill entries: grid-stride over the view's pool (blockIdx.y walks the views), one thread per fill edge = the two
+// entries (j <- k), (k <- j) it left in adjacent slots (reservations are even, so pairs never straddle); if both
+// endpoints are alive each entry goes to the tail of its owner's staging segment, filled from the end backwards (the
+// front is where the alive base entries of a merge-path vertex go; cursor[v] counts the fills of v)
+constexpr long long MAX_GRID_Y = 65535;   // CUDA's limit on gridDim.y: a call may have more views
 __global__ void __launch_bounds__(256) k_emit_scatter(SchurParams P) {
     if (run_failed(P)) return;
-    const int view = blockIdx.y;
-    const size_t vb = (size_t)view * (size_t)P.n;
     const long long t0 = (long long)blockIdx.x * blockDim.x + threadIdx.x, nt = (long long)gridDim.x * blockDim.x;
-    long long used = (long long)P.pool_cursor[view];
-    if (used > P.pool_cap) used = P.pool_cap;
-    const int4* pool = P.pool + (size_t)view * (size_t)P.pool_cap;
-    for (long long e = 2 * t0; e + 1 < used; e += 2 * nt) {
-        const int4 e0 = __ldcs(pool + e);        // {k, w, next, j}
-        if (e0.w < 0) continue;                  // tombstones come in pairs as well
-        const int j = e0.w, k = e0.x;
-        if (P.state[vb + j] == 2 || P.state[vb + k] == 2) continue;
-        const long long p0 = P.rawoff[vb + j + 1] - 1 - atomicAdd(cursor_of(P) + vb + j, 1);
-        const long long p1 = P.rawoff[vb + k + 1] - 1 - atomicAdd(cursor_of(P) + vb + k, 1);
-        if (p0 >= 0 && p1 >= 0 && p0 < P.raw_cap && p1 < P.raw_cap) {
-            P.raw[p0] = ((uint64_t)(uint32_t)k << 32) | (uint64_t)(uint32_t)e0.y;
-            P.raw[p1] = ((uint64_t)(uint32_t)j << 32) | (uint64_t)(uint32_t)e0.y;
-        } else {
-            set_status(P, 6);
+    for (int view = blockIdx.y; view < P.V; view += gridDim.y) {
+        const size_t vb = (size_t)view * (size_t)P.n;
+        long long used = (long long)P.pool_cursor[view];
+        if (used > P.pool_cap) used = P.pool_cap;
+        const int4* pool = P.pool + (size_t)view * (size_t)P.pool_cap;
+        for (long long e = 2 * t0; e + 1 < used; e += 2 * nt) {
+            const int4 e0 = __ldcs(pool + e);        // {k, w, next, j}
+            if (e0.w < 0) continue;                  // tombstones come in pairs as well
+            const int j = e0.w, k = e0.x;
+            if (P.state[vb + j] == 2 || P.state[vb + k] == 2) continue;
+            const long long p0 = P.rawoff[vb + j + 1] - 1 - atomicAdd(cursor_of(P) + vb + j, 1);
+            const long long p1 = P.rawoff[vb + k + 1] - 1 - atomicAdd(cursor_of(P) + vb + k, 1);
+            if (p0 >= 0 && p1 >= 0 && p0 < P.raw_cap && p1 < P.raw_cap) {
+                P.raw[p0] = ((uint64_t)(uint32_t)k << 32) | (uint64_t)(uint32_t)e0.y;
+                P.raw[p1] = ((uint64_t)(uint32_t)j << 32) | (uint64_t)(uint32_t)e0.y;
+            } else {
+                set_status(P, 6);
+            }
         }
     }
 }
@@ -820,7 +822,8 @@ cudaError_t launch_emit_count(const SchurParams& P, long long* total_dev, cudaSt
         long long bx = (work + 256 * 4 - 1) / (256 * 4);
         if (bx < 1) bx = 1;
         if (bx > 148 * 8) bx = 148 * 8;
-        k_emit_scatter<<<dim3((unsigned)bx, (unsigned)P.V), 256, 0, stream>>>(P);
+        const long long by = P.V < MAX_GRID_Y ? P.V : MAX_GRID_Y;
+        k_emit_scatter<<<dim3((unsigned)bx, (unsigned)by), 256, 0, stream>>>(P);
         DBG_SYNC("k_emit_scatter");
         bx = ((long long)P.V * ((P.n + 31) / 32) + 7) / 8;   // one warp per 32 vertices of a view
         if (bx < 1) bx = 1;

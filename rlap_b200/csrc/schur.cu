@@ -274,6 +274,9 @@ __device__ __forceinline__ bool push_fill(const PT& P, int view, size_t vb, int4
     if (!(w > 0.f)) {  // underflowed fill: leave two tombstones so that the pool can be read linearly
         pool[slot] = make_int4(-1, 0, -1, -1);
         pool[slot + 1] = make_int4(-1, 0, -1, -1);
+        // the callers count a star's fills before they are sampled: take this one back (the stat counts fill edges,
+        // as the lane path and the oracle do; the group's sum stays exact modulo 2^64)
+        atomicAdd(P.stats + ST_FILLS, ~0ull);
         return false;
     }
     {   // both list heads are exchanged before either entry is written: the two round trips overlap
