@@ -30,7 +30,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     flags = list(NVCC_FLAGS)
     if os.environ.get("RLAP_DEBUG_BUILD"):   # profiling build: phase wait timers, RLAP_GROUPS / RLAP_DEBUG_SYNC knobs
         flags.append("-DRLAP_DEBUG")
-    flags += os.environ.get("RLAP_NVCC_EXTRA", "").split()     # experiments: e.g. -DRLAP_LVL_AHEAD=2
+    flags += os.environ.get("RLAP_NVCC_EXTRA", "").split()     # experiments: extra nvcc flags
     # one nvcc per translation unit, side by side (the elimination kernel is compiled once per mode: most of the time)
     from concurrent.futures import ThreadPoolExecutor
     os.makedirs(OBJ_DIR, exist_ok=True)

@@ -41,26 +41,44 @@ __global__ void k_emit_prep(SchurParams P) {
     cursor_of(P)[idx] = 0;
 }
 
+// Merge-path segments are listed by size class in dense lists (the low-list buffers of the elimination are free by
+// now): a hub-heavy stretch of vertex ids (the old vertices of a preferential-attachment graph) would otherwise hand
+// all its big segments to the few warps that own that stretch.
+constexpr int CAP_REGS = 512;   // largest segment sorted in registers
+constexpr int N_CLASS = 7;
+// classes 6, 0..3: at most 32 / 64 / 128 / 256 / 512 entries (register sort, k_emit_sort_mid), 4: at most CAP_CTA
+// (k_emit_sort_block), 5: above (k_emit_sort_big, or a scratch slot in k_emit_sort_block)
+__host__ __device__ constexpr int size_class(int lv) {
+    return lv <= 32 ? 6 : lv <= 64 ? 0 : lv <= 128 ? 1 : lv <= 256 ? 2 : lv <= CAP_REGS ? 3 : lv <= CAP_CTA ? 4 : 5;
+}
+__device__ __forceinline__ unsigned int* class_list(const SchurParams& P, int c) {
+    const size_t VN = (size_t)P.V * (size_t)P.n;
+    if (c == 0) return P.wl;
+    if (c == 1) return P.wl + VN;
+    if (c == 5) return P.dl;
+    if (c == 6) return P.low + (size_t)3 * (VN + 16);
+    return P.low + (size_t)(c - 2) * (VN + 16);
+}
+__device__ __forceinline__ int* class_tail(const SchurParams& P, int c) { return P.ctr + CTR_EMIT_C0 + c; }
+
 // Base entries of the survivors on the merge path (cursor == MERGE_PATH): a warp per vertex walks its
 // (neighbour-ascending) CSR row and writes the entries whose neighbour is alive to the front of the vertex's staging
 // segment, in order and without atomics. The vertices come from the size-class lists k_emit_fsort built (one virtual
 // list: the classes back to back) - about 1 % of the survivors, mostly hubs; a sweep over every vertex of every view
 // spent 197 M warp instructions (0.35 ms per 64 arxiv views) finding them.
 constexpr int MERGE_PATH = -1;
-constexpr int N_CLASS_FWD = 7;   // = N_CLASS (declared with the lists below)
-__device__ __forceinline__ unsigned int* class_list(const SchurParams& P, int c);
 __global__ void __launch_bounds__(256) k_emit_base(SchurParams P) {
     if (run_failed(P)) return;
     const int gw = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     const int nw = (int)(((long long)gridDim.x * blockDim.x) >> 5);
     const int lane = threadIdx.x & 31;
-    int tails[N_CLASS_FWD], total = 0;
+    int tails[N_CLASS], total = 0;
 #pragma unroll
-    for (int c = 0; c < N_CLASS_FWD; c++) { tails[c] = P.ctr[CTR_EMIT_C0 + c]; total += tails[c]; }
+    for (int c = 0; c < N_CLASS; c++) { tails[c] = P.ctr[CTR_EMIT_C0 + c]; total += tails[c]; }
     for (int it = gw; it < total; it += nw) {
         int c = 0, r = it;
 #pragma unroll
-        for (int k = 0; k < N_CLASS_FWD - 1; k++) {
+        for (int k = 0; k < N_CLASS - 1; k++) {
             if (c == k && r >= tails[k]) { r -= tails[k]; c = k + 1; }
         }
         const unsigned int idx = class_list(P, c)[r];
@@ -111,16 +129,15 @@ __global__ void __launch_bounds__(256) k_emit_scatter(SchurParams P) {
     }
 }
 
-// sort + merge a staged star (shared memory or scratch) and write the merged entries back to the
-// start of the vertex's raw segment, neighbours ascending
-template <bool CTA>
+// sort + merge a staged star (shared memory or scratch) with the whole thread block and write the merged entries back
+// to the start of the vertex's raw segment, neighbours ascending
 __device__ void emit_sort_staged(const SchurParams& P, size_t idx, StarBuf sb, CtaScratch* cs) {
-    const int gs = g_size<CTA>(), r = g_rank<CTA>(), lane = threadIdx.x & 31;
+    const int gs = (int)blockDim.x, r = (int)threadIdx.x, lane = threadIdx.x & 31;
     const int lraw = rawcnt_of(P)[idx];
     const long long off = P.rawoff[idx];
     if (lraw > sb.cap) {
         if (r == 0) { set_status(P, 6); P.outcnt[idx] = 0; }
-        g_sync<CTA>();
+        __syncthreads();
         return;
     }
     uint32_t wmaxb = 0;
@@ -130,18 +147,18 @@ __device__ void emit_sort_staged(const SchurParams& P, size_t idx, StarBuf sb, C
         sb.A[i] = a;
         if (i < lraw) wmaxb = max(wmaxb, (uint32_t)a);
     }
-    g_sync<CTA>();
-    g_bitonic_sort_keys<CTA>(sb.A, P2);
+    __syncthreads();
+    g_bitonic_sort_keys<true>(sb.A, P2);
     // multi-edges are rare among survivors: look for one before paying for the fixed-point merge
     int dup = 0;
     for (int i = r + 1; i < lraw; i += gs) dup |= (a_nbr(sb.A[i]) == a_nbr(sb.A[i - 1]));
-    dup = CTA ? __syncthreads_or(dup) : __any_sync(RLAP_FULL_MASK, dup);
+    dup = __syncthreads_or(dup);
     int L = lraw;
     if (dup) {
-        wmaxb = g_max_u32<CTA>(wmaxb, cs);
-        g_sync<CTA>();
+        wmaxb = g_max_u32<true>(wmaxb, cs);
+        __syncthreads();
         const int shift = star_shift(__uint_as_float(wmaxb), lraw);
-        L = star_merge_sorted<CTA>(sb, lraw, shift, cs);
+        L = star_merge_sorted<true>(sb, lraw, shift, cs);
     }
     int carry = 0;
     for (int base = 0; base < lraw; base += gs) {
@@ -150,23 +167,18 @@ __device__ void emit_sort_staged(const SchurParams& P, size_t idx, StarBuf sb, C
         bool keep = (i < lraw) && !a_dead(a);
         unsigned m = __ballot_sync(RLAP_FULL_MASK, keep);
         int pos = __popc(m & ((1u << lane) - 1u));
-        if (CTA) {
-            int w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-            __syncthreads();
-            if (lane == 0) cs->wsum[w] = (unsigned long long)__popc(m);
-            __syncthreads();
-            int add = 0, tot = 0;
-            for (int k = 0; k < nw; k++) { int c = (int)cs->wsum[k]; if (k < w) add += c; tot += c; }
-            pos += add + carry;
-            carry += tot;
-        } else {
-            pos += carry;
-            carry += __popc(m);
-        }
+        const int w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+        __syncthreads();
+        if (lane == 0) cs->wsum[w] = (unsigned long long)__popc(m);
+        __syncthreads();
+        int add = 0, tot = 0;
+        for (int k = 0; k < nw; k++) { int c = (int)cs->wsum[k]; if (k < w) add += c; tot += c; }
+        pos += add + carry;
+        carry += tot;
         if (keep) P.raw[off + pos] = a;
     }
     if (r == 0) P.outcnt[idx] = L;
-    g_sync<CTA>();
+    __syncthreads();
 }
 
 // A warp sorts one segment of up to 32 * R entries in registers (element e = r * 32 + lane), merges the runs of
@@ -264,26 +276,6 @@ __device__ void emit_sort_regs(const SchurParams& P, size_t idx, int lv, long lo
     }
     if (lane == 0) P.outcnt[idx] = rowbase;
 }
-
-// Segments of more than 32 entries are listed by size class in dense lists (the low-list buffers of the elimination
-// are free by now): a hub-heavy stretch of vertex ids (the old vertices of a preferential-attachment graph) would
-// otherwise hand all its big segments to the few warps that own that stretch.
-constexpr int CAP_REGS = 512;   // largest segment sorted in registers
-constexpr int N_CLASS = 7;
-static_assert(N_CLASS == N_CLASS_FWD, "k_emit_base walks every class list");
-// classes 0..3: 64 / 128 / 256 / 512 entries (register sort), 4: <= CAP_CTA, 5: above, 6: <= 32
-__device__ __forceinline__ unsigned int* class_list(const SchurParams& P, int c) {
-    const size_t VN = (size_t)P.V * (size_t)P.n;
-    if (c == 0) return P.wl;
-    if (c == 1) return P.wl + VN;
-    if (c == 5) return P.dl;
-    if (c == 6) return P.low + (size_t)3 * (VN + 16);
-    return P.low + (size_t)(c - 2) * (VN + 16);
-}
-__device__ __forceinline__ int size_class(int lv) {
-    return lv <= 32 ? 6 : lv <= 64 ? 0 : lv <= 128 ? 1 : lv <= 256 ? 2 : lv <= CAP_REGS ? 3 : lv <= CAP_CTA ? 4 : 5;
-}
-__device__ __forceinline__ int* class_tail(const SchurParams& P, int c) { return P.ctr + CTR_EMIT_C0 + c; }
 
 constexpr int CAP_BIG = 12288;   // largest segment sorted in the shared memory of one SM (k_emit_sort_big)
 
@@ -426,35 +418,12 @@ __global__ void __launch_bounds__(256) k_emit_fsort(SchurParams P) {
     }
 }
 
-// merge path, segments of at most 32 entries: one warp each, one entry per lane
-__global__ void __launch_bounds__(256) k_emit_sort_small(SchurParams P) {
-    const int gw = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
-    const int nw = (int)(((long long)gridDim.x * blockDim.x) >> 5);
-    const int lane = threadIdx.x & 31;
-    const unsigned lt = (1u << lane) - 1u;
-    const int end = *class_tail(P, 6);
-    const unsigned int* list = class_list(P, 6);
-    for (int it = gw; it < end; it += nw) {
-        const unsigned int idx = list[it];
-        const int lv = rawcnt_of(P)[idx];
-        const long long off = P.rawoff[idx];
-        uint64_t a = lane < lv ? P.raw[off + lane] : RLAP_PAD_A;
-        a = warp_sort_u64(a);
-        unsigned long long q;
-        int shift;
-        const unsigned hmask = warp_merge_sorted(a, q, shift, false);
-        if ((hmask >> lane) & 1u) P.raw[off + __popc(hmask & lt)] = a;
-        if (lane == 0) P.outcnt[idx] = __popc(hmask);
-    }
-}
-
-// segments of 33..512 entries: one warp each, registers only. One kernel per size class (64, 128, 256, 512 entries =
-// 2, 4, 8, 16 keys per lane) so that the small classes, which hold most segments, run at their own register budget.
-// The list entry carries the class in its two top bits (V * n < 2^30); a warp takes 32 entries, reads their
-// counts and offsets in one go and sorts the ones of its class.
+// segments of at most 512 entries: one warp each, registers only. One kernel per size class (32, 64, 128, 256, 512
+// entries = 1, 2, 4, 8, 16 keys per lane) so that the small classes, which hold most segments, run at their own
+// register budget.
 template <int R>
 __global__ void __launch_bounds__(256, (R <= 4 ? 4 : 2)) k_emit_sort_mid(SchurParams P) {
-    constexpr int CLS = (R == 2 ? 0 : R == 4 ? 1 : R == 8 ? 2 : 3);
+    constexpr int CLS = size_class(32 * R);
     const int gw = (int)(((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     const int nw = (int)(((long long)gridDim.x * blockDim.x) >> 5);
     const int end = *class_tail(P, CLS);
@@ -471,7 +440,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, 2) k_emit_sort_block(SchurParam
     const int end = *class_tail(P, 4);
     const unsigned int* list = class_list(P, 4);
     for (int it = (int)blockIdx.x; it < end; it += (int)gridDim.x) {
-        emit_sort_staged<true>(P, list[it], cta_buf(smem), &cs);
+        emit_sort_staged(P, list[it], cta_buf(smem), &cs);
         __syncthreads();
     }
     // segments beyond the shared memory of an SM: the NSLOT blocks that own a global scratch slot
@@ -481,7 +450,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, 2) k_emit_sort_block(SchurParam
         for (int it = (int)blockIdx.x; it < end5; it += NSLOT) {
             const unsigned int idx = list5[it];
             if (rawcnt_of(P)[idx] <= CAP_BIG) continue;
-            emit_sort_staged<true>(P, idx, scratch_buf(P), &cs);
+            emit_sort_staged(P, idx, scratch_buf(P), &cs);
             __syncthreads();
         }
     }
@@ -499,7 +468,7 @@ __global__ void __launch_bounds__(BLOCK_THREADS, 1) k_emit_sort_big(SchurParams 
     for (int it = (int)blockIdx.x; it < end; it += (int)gridDim.x) {
         const unsigned int idx = list[it];
         if (rawcnt_of(P)[idx] > CAP_BIG) continue;
-        emit_sort_staged<true>(P, idx, sb, &cs);
+        emit_sort_staged(P, idx, sb, &cs);
         __syncthreads();
     }
 }
@@ -845,7 +814,7 @@ cudaError_t launch_emit_count(const SchurParams& P, long long* total_dev, cudaSt
         e = cudaStreamWaitEvent(aux[i], aux_ev[6], 0);
         if (e != cudaSuccess) return e;
     }
-    k_emit_sort_small<<<148 * 4, 256, 0, stream>>>(P);
+    k_emit_sort_mid<1><<<148 * 4, 256, 0, stream>>>(P);
     k_emit_sort_mid<2><<<148 * 4, 256, 0, aux[0]>>>(P);
     k_emit_sort_mid<4><<<148 * 4, 256, 0, aux[1]>>>(P);
     k_emit_sort_mid<8><<<148 * 2, 256, 0, aux[2]>>>(P);

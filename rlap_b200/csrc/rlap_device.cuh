@@ -128,7 +128,6 @@ struct CtaScratch {
     unsigned long long wsum[32];
     unsigned long long carry;
     int icount;
-    int ibcast[4];
 };
 
 __device__ __forceinline__ unsigned long long warp_incl_scan_u64(unsigned long long v) {

@@ -20,12 +20,6 @@
 #include "scan.cuh"
 #include "star.cuh"
 
-// keys past the bucket key that a rescan lists as well (see phase B2). Measured on the arxiv shape, 64 views: 0 -> 5.15 ms,
-// 1 -> 5.26 ms, 2 -> 5.61 ms for k_eliminate: the longer low lists cost more than the rescans they save.
-#ifndef RLAP_LVL_AHEAD
-#define RLAP_LVL_AHEAD 0
-#endif
-
 namespace rlap {
 
 __device__ __forceinline__ int graph_of(const SchurParams& P, int v) { return P.gid ? __ldg(P.gid + v) : 0; }
@@ -455,29 +449,23 @@ __device__ void eliminate_star(const PT& P, const RoundCtx& rc, int view, int v,
     g_sync<CTA>();
 }
 
-// Register-resident elimination: a tile of W lanes (8, 16 or 32) holds one star, one entry per lane, and
-// the 32 / W tiles of a warp run in lock step (all shuffles are tile-wide). `idx` is the tile's work
-// item (uniform inside the tile) or 0xffffffff for an idle tile. The caller has already read the star's CSR
-// bounds (b, nb) and walked its fill list into shared memory (`fills`, nfill entries), and guarantees
-// nb + nfill <= W: the raw list always fits, nothing is retried.
+// Register-resident elimination: the warp holds one star, one entry per lane. `idx` is the warp's work item, warp
+// uniform and always a real star. The caller has already read the star's CSR bounds (b, nb) and walked its fill list
+// into shared memory (`fills`, nfill entries), and guarantees nb + nfill <= 32: the raw list always fits, nothing is
+// retried.
 // `slot0` / `nslots`: pool slots reserved for this star by the caller (an upper bound, 2 per possible fill).
-template <int W, class PT>
-__device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned int idx, int b, int nb,
+template <class PT>
+__device__ void eliminate_star_regs(const PT& P, const RoundCtx& rc, unsigned int idx, int b, int nb,
                                     const uint64_t* fills, int nfill, long long slot0, int nslots, int M,
                                     LocalStats* ls, PendingPush& pend, LowAppender& la) {
-    typedef Tile<W> T;
-    const int tl = T::tl();
-    const bool active = idx != 0xffffffffu;
-    const int view = active ? (int)(idx / (unsigned)P.n) : 0, v = active ? (int)(idx % (unsigned)P.n) : 0;
+    const int tl = threadIdx.x & 31;
+    const int view = (int)(idx / (unsigned)P.n), v = (int)(idx % (unsigned)P.n);
     const size_t vb = (size_t)view * (size_t)P.n;
     const uint32_t view_id = P.view_base + (uint32_t)view;
     int4* pool = P.pool + (size_t)view * (size_t)P.pool_cap;
-    const bool fail = false;
     uint64_t a = RLAP_PAD_A;
-    if (active) {
-        if (tl < nb) a = pack_a((uint32_t)__ldg(P.col + b + tl), __ldg(P.w + b + tl));
-        else if (tl - nb < nfill) a = fills[tl - nb];
-    }
+    if (tl < nb) a = pack_a((uint32_t)__ldg(P.col + b + tl), __ldg(P.w + b + tl));
+    else if (tl - nb < nfill) a = fills[tl - nb];
     bool dead = false;
     // dead test on the neighbour's (live, head) record: the sector is the one its live counter and list head are
     // updated in further down
@@ -486,20 +474,19 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
     pend.flush(la);
     if (dead) a = RLAP_PAD_A;
     __syncwarp();
-    const bool go = active && !fail;
-    a = T::sort_u64(a);
+    a = warp_sort_u64(a);
     const bool rawvalid = a != RLAP_PAD_A;         // raw live entry (multi-edge duplicates included)
     const int rawnbr = (int)a_nbr(a);
-    const int lraw = __popc(T::ballot(rawvalid));
+    const int lraw = __popc(__ballot_sync(RLAP_FULL_MASK, rawvalid));
     unsigned long long q;
     int shift;
     int mult;
-    const unsigned hmask = T::merge_sorted(a, q, shift, true, mult);
+    const unsigned hmask = warp_merge_sorted(a, q, shift, mult);
     const int L = __popc(hmask);
     // live counters: a neighbour loses its entries to v (all `mult` of them) and gains one entry per fill it
     // receives. The extra multiplicity goes now, the rest is netted per merged neighbour after sampling.
     bool cross0 = false;
-    if (go && ((hmask >> tl) & 1u) && mult > 1) {
+    if (((hmask >> tl) & 1u) && mult > 1) {
         const int old = atomicSub(live_p(P, vb + rawnbr), mult - 1);
         cross0 = old > M && old - (mult - 1) <= M;
     }
@@ -509,10 +496,9 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
     const int on = coarsen ? 2 : P.o_n;
     uint64_t key = ~0ull, tie = 0;
     // asc / desc ties among more than 16 merged neighbours: position in the arrangement std::sort's partition loop
-    // leaves (star.cuh). Only a 32-lane tile (one star per warp: the branch is warp uniform) can hold that many. The
-    // tile's own FCAP staged fills (128 bytes, read into `a` above) serve as its workspace.
+    // leaves (star.cuh). The warp's FCAP staged fills (128 bytes, read into `a` above) serve as its workspace.
     uint64_t tiepos = 0;
-    if (W == 32 && !full && on != 2 && L > 16)
+    if (!full && on != 2 && L > 16)
         tiepos = (on == 1) ? warp_tie_order<true>(q, hmask, (uint8_t*)const_cast<uint64_t*>(fills))
                            : warp_tie_order<false>(q, hmask, (uint8_t*)const_cast<uint64_t*>(fills));
     if (live) {
@@ -529,51 +515,50 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
         q = 0;
         tie = ~0ull;   // padding sorts after every live entry, also after one whose key is ~0 (q = 0 under desc)
     }
-    if (W == 32) T::sort_ktaq(key, tie, a, q);   // only a 32-lane tile can hold more than 16 neighbours
-    else T::sort_kaq(key, a, q);
+    warp_sort_ktaq(key, tie, a, q);
     // o_v = random: the entry's neighbour still to be eliminated? and its rank, read here for all lanes at once instead
     // of by every push (a neighbour of the vertex being eliminated cannot change state inside this round)
     bool pend_mine = false;
     int rank_mine = 0;
-    if (P.o_v == 0 && go && a != RLAP_PAD_A) {
+    if (P.o_v == 0 && a != RLAP_PAD_A) {
         pend_mine = ldcg_u8(P.state + vb + a_nbr(a)) == 1;
         rank_mine = ldcg_i32(P.rank + vb + a_nbr(a));
     }
-    const unsigned long long C = T::incl_scan(q);
-    const unsigned long long S = __shfl_sync(RLAP_FULL_MASK, C, (L > 0 ? L - 1 : 0), W);
+    const unsigned long long C = warp_incl_scan_u64(q);
+    const unsigned long long S = __shfl_sync(RLAP_FULL_MASK, C, (L > 0 ? L - 1 : 0));
     const long long nf = (L < 1) ? 0 : (full ? (long long)L * (L - 1) / 2 : (long long)(L - 1));
     const bool ovf = nslots > 0 && slot0 + nslots > P.pool_cap;
-    if (go && ovf && tl == 0) set_status(P, 5);
-    const bool emit = go && nf > 0 && !ovf;
+    if (ovf && tl == 0) set_status(P, 5);
+    const bool emit = nf > 0 && !ovf;
     // reserved but unused slots (multi-edges merged): tombstones, the pool is read linearly at emission
-    if (go && !ovf)
-        for (long long u = 2 * nf + tl; u < nslots; u += W) pool[slot0 + u] = make_int4(-1, 0, -1, -1);
+    if (!ovf)
+        for (long long u = 2 * nf + tl; u < nslots; u += 32) pool[slot0 + u] = make_int4(-1, 0, -1, -1);
     int delta = -1;   // net change of live[neighbour] for the merged neighbour held by this lane
     if (full) {
         const double Sf = __dmul_rn(__ull2double_rn(S), pow2d(-shift));
-        for (int b2 = 1; b2 < W; b2++) {
-            const uint64_t eb = __shfl_sync(RLAP_FULL_MASK, a, b2, W);
+        for (int b2 = 1; b2 < 32; b2++) {
+            const uint64_t eb = __shfl_sync(RLAP_FULL_MASK, a, b2);
             bool done = false;
             if (emit && b2 < L && tl < b2) {
                 float w = __double2float_rn(__ddiv_rn(__dmul_rn((double)a_w(a), (double)a_w(eb)), Sf));
                 long long off = (long long)tl * (2LL * L - tl - 1) / 2;
                 done = push_fill<false>(P, view, vb, pool, (int)a_nbr(a), (int)a_nbr(eb), w, slot0 + 2 * (off + (b2 - tl - 1)));
             }
-            unsigned dm = T::ballot(done);
+            unsigned dm = __ballot_sync(RLAP_FULL_MASK, done);
             if (done) delta++;
             if (tl == b2) delta += __popc(dm);
         }
     } else if (coarsen) {
         uint4 x = philox4x32_10(P.k0, P.k1, (uint32_t)v, 0xffffffffu, view_id, TAG_PICK);
         unsigned long long u = ((unsigned long long)x.x << 32) | (unsigned long long)x.y;
-        int koff = T::upper_bound(C, L, __umul64hi(u, S));
+        int koff = warp_upper_bound(C, L, __umul64hi(u, S));
         if (koff >= L) koff = L - 1;
         if (koff < 0) koff = 0;
-        const uint64_t ek = __shfl_sync(RLAP_FULL_MASK, a, koff, W);
+        const uint64_t ek = __shfl_sync(RLAP_FULL_MASK, a, koff);
         int dep = -1;
         if (P.o_v == 0) {
-            const bool pk = __shfl_sync(RLAP_FULL_MASK, pend_mine, koff, W);
-            const int rkk = __shfl_sync(RLAP_FULL_MASK, rank_mine, koff, W);
+            const bool pk = __shfl_sync(RLAP_FULL_MASK, pend_mine, koff);
+            const int rkk = __shfl_sync(RLAP_FULL_MASK, rank_mine, koff);
             dep = (pend_mine && pk) ? (rank_mine < rkk ? 1 : 2) : 0;
         }
         bool done = false;
@@ -583,7 +568,7 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
             int sl = tl < koff ? tl : tl - 1;
             done = push_fill<false>(P, view, vb, pool, (int)a_nbr(a), (int)a_nbr(ek), w, slot0 + 2LL * sl, &pend, dep);
         }
-        unsigned dm = T::ballot(done);
+        unsigned dm = __ballot_sync(RLAP_FULL_MASK, done);
         if (done) delta++;
         if (tl == koff) delta += __popc(dm);
     } else {
@@ -595,14 +580,14 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
             unsigned long long u = ((unsigned long long)x.x << 32) | (unsigned long long)x.y;
             rr = C + __umul64hi(u, rem);
         }
-        int koff = T::upper_bound(C, L, rr);
+        int koff = warp_upper_bound(C, L, rr);
         if (koff >= L) koff = L - 1;
         if (koff < 0) koff = 0;
-        const uint64_t ek = __shfl_sync(RLAP_FULL_MASK, a, koff, W);
+        const uint64_t ek = __shfl_sync(RLAP_FULL_MASK, a, koff);
         int dep = -1;
         if (P.o_v == 0) {
-            const bool pk = __shfl_sync(RLAP_FULL_MASK, pend_mine, koff, W);
-            const int rkk = __shfl_sync(RLAP_FULL_MASK, rank_mine, koff, W);
+            const bool pk = __shfl_sync(RLAP_FULL_MASK, pend_mine, koff);
+            const int rkk = __shfl_sync(RLAP_FULL_MASK, rank_mine, koff);
             dep = (pend_mine && pk) ? (rank_mine < rkk ? 1 : 2) : 0;
         }
         if (emit && act) {
@@ -619,12 +604,12 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
     __syncwarp();
     // neighbours whose live counter crossed the segment's level downwards join the next round's low list; the test
     // on the value the atomic returns is left to the next flush of `pend`
-    if (go && tl < L && delta != 0) {
+    if (tl < L && delta != 0) {
         const int old = atomicAdd(live_p(P, vb + (int)a_nbr(a)), delta);
         if (delta < 0) { pend.lo_old = old; pend.lo_M = M; pend.lo_lim = M - delta; pend.lo_idx = (unsigned int)(vb + (size_t)a_nbr(a)); }
     }
     la.push(cross0, (unsigned int)(vb + (size_t)rawnbr));
-    if (go && rawvalid) {
+    if (rawvalid) {
         if (P.o_v == 0 && ldcg_u8(P.state + vb + rawnbr) == 1) {
             int old = atomicSub(P.blk + vb + rawnbr, 1);
             if (old == 1) {
@@ -633,7 +618,7 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
             }
         }
     }
-    if (go && tl == 0) {
+    if (tl == 0) {
         ls->fills += (unsigned long long)(ovf ? 0 : nf);
         ls->maxstar = max(ls->maxstar, L);
         ls->raw += (unsigned long long)lraw;
@@ -648,11 +633,11 @@ __device__ void eliminate_star_tile(const PT& P, const RoundCtx& rc, unsigned in
 // lane stars: one THREAD per star
 // ---------------------------------------------------------------------------------------------
 // A star with at most LCAP live entries and no multi-edge is gathered, ordered, sampled and pushed by a single lane
-// out of its own shared-memory slot. The register tiles keep 4 (8 lanes) or 2 (16 lanes) dependent chains of memory
-// round trips in flight per warp and spend a warp-wide sorting network on 7..13 entries; here a warp keeps 32 chains
-// in flight and every lane runs a short insertion sort over an almost sorted list. The arithmetic is the keyed
-// specification's (DESIGN.md §3.3) to the bit: same fixed point, same tie rules (a star of at most 16 neighbours
-// breaks asc / desc ties by neighbour id), same Philox counters, same IEEE double weight formula.
+// out of its own shared-memory slot: a warp keeps 32 dependent chains of memory round trips in flight, and every lane
+// runs a short insertion sort over an almost sorted list instead of a warp-wide sorting network (DESIGN.md §4, "Lane
+// stars"). The arithmetic is the keyed specification's (DESIGN.md §3.3) to the bit: same fixed point, same tie rules
+// (a star of at most 16 neighbours breaks asc / desc ties by neighbour id), same Philox counters, same IEEE double
+// weight formula.
 // Stars the lane cannot finish alone (a multi-edge, which needs the summed fixed-point weight of the run; two equal
 // 32-bit shuffle keys, which need the full 64-bit key; more entries than announced) are handed to the cooperative
 // path untouched: the lane returns false before it has modified anything.
@@ -921,38 +906,6 @@ __device__ bool eliminate_star_lane(const PT& P, const RoundCtx& rc, unsigned in
 constexpr int FCAP = 16;  // fill entries per item that the chunk prologue stages in shared memory (32 x FCAP words = the lane slots)
 static_assert(FCAP * sizeof(uint64_t) >= 96, "warp_tie_order keeps 3 x 32 bytes in a tile's staged-fill slot");
 
-// Run one tier: the items whose bit is set in `mask` (lane i holds item i of the warp's chunk) are handed
-// to the 32 / W tiles of the warp, 32 / W at a time.
-template <int W, class PT>
-__device__ void run_tier(const PT& P, const RoundCtx& rc, unsigned mask, unsigned int my_idx, int my_b,
-                         int my_nb, int my_nfill, const uint64_t* fbuf, long long my_slot0, int my_nslots, int my_M,
-                         LocalStats* ls, PendingPush& pend, LowAppender& la) {
-    constexpr int TPW = 32 / W;
-    const int lane = threadIdx.x & 31;
-    const int tile = lane / W;
-    while (mask) {
-        // tile t takes the t-th pending item (lowest set bits first)
-        unsigned rest = mask;
-        unsigned src = 0xffffffffu;
-#pragma unroll
-        for (int t = 0; t < TPW; t++) {
-            const unsigned took = rest ? (unsigned)(__ffs(rest) - 1) : 0xffffffffu;
-            if (t == tile) src = took;
-            rest &= rest - 1;          // 0 & anything stays 0
-        }
-        const int sl = (int)(src & 31);
-        unsigned int idx = __shfl_sync(RLAP_FULL_MASK, my_idx, sl);
-        const int b = __shfl_sync(RLAP_FULL_MASK, my_b, sl), nb = __shfl_sync(RLAP_FULL_MASK, my_nb, sl);
-        const int nfill = __shfl_sync(RLAP_FULL_MASK, my_nfill, sl);
-        const long long sl0 = __shfl_sync(RLAP_FULL_MASK, my_slot0, sl);
-        const int nsl = __shfl_sync(RLAP_FULL_MASK, my_nslots, sl);
-        const int M = __shfl_sync(RLAP_FULL_MASK, my_M, sl);
-        if (src == 0xffffffffu) idx = 0xffffffffu;
-        eliminate_star_tile<W>(P, rc, idx, b, nb, fbuf + sl * FCAP, nfill, sl0, nsl, M, ls, pend, la);
-        mask = rest;
-    }
-}
-
 // shared memory of the elimination phase, per warp: the lane slots (LCAP x 32 entries, plus 32-bit shuffle keys when
 // the neighbour order is random), overlaid by the staging area of the register tiles and the star buffer of the
 // shared-memory path, which run after the lane stars of a chunk
@@ -977,8 +930,8 @@ __device__ __forceinline__ StarBuf warp_region_buf(const PT& P, uint64_t* smem) 
 // live entries are eliminated by their lane alone (eliminate_star_lane); up to 32 raw entries by the warp as a
 // register tile; up to CAP_WARP by the warp in shared memory; big stars go to the block phase.
 template <class PT>
-__device__ void run_warp_items(const PT& P, const RoundCtx& rc, uint64_t* smem, CtaScratch* cs, int* next,
-                               int start, int end, LocalStats* ls, LowAppender& la) {
+__device__ void run_warp_items(const PT& P, const RoundCtx& rc, uint64_t* smem, CtaScratch* cs, int start, int end,
+                               LocalStats* ls, LowAppender& la) {
     const int nw = (int)((P.gblocks * blockDim.x) >> 5);
     const int lane = threadIdx.x & 31;
     StarBuf sb = warp_region_buf(P, smem);
@@ -991,7 +944,6 @@ __device__ void run_warp_items(const PT& P, const RoundCtx& rc, uint64_t* smem, 
     // All warps of the launch (a view group) fetch chunks of the round's work list from one global cursor, with a
     // guided size: 1 / (2 x warps) of what is left, at least 8 and at most 32 items. A stale read of the cursor only
     // changes a chunk size.
-    (void)next;
     const bool full = P.full;
     enum { K_NONE = 0, K_LANE = 1, K_TILE = 2, K_SMEM = 3 };
     // pool slots are reserved once per chunk and tier: 2 per possible fill (L <= live), one atomic per view present in
@@ -1135,9 +1087,21 @@ __device__ void run_warp_items(const PT& P, const RoundCtx& rc, uint64_t* smem, 
             if (kind == K_TILE && lv >= 2) nslots = full ? lv * (lv - 1) : 2 * (lv - 1);
             const Resv rv = reserve_issue(nslots, view);
             const long long slot0 = reserve_finish(rv, nslots);
-            const unsigned m32 = __ballot_sync(RLAP_FULL_MASK, kind == K_TILE);
+            // The & 31 changes no value (mt != 0). It steers ptxas, CUDA 12.9: without it k_eliminate<0, 0 or 1, false>
+            // spill 128 / 104 bytes instead of 88 / 80.
+            unsigned mt = __ballot_sync(RLAP_FULL_MASK, kind == K_TILE);
             PendingPush pend;
-            run_tier<32>(P, rc, m32, idx, b, nb, nfill, fbuf, slot0, nslots, M, ls, pend, la);
+            while (mt) {
+                const int k = (__ffs(mt) - 1) & 31;
+                mt &= mt - 1;
+                const unsigned int kidx = __shfl_sync(RLAP_FULL_MASK, idx, k);
+                const int kb = __shfl_sync(RLAP_FULL_MASK, b, k), knb = __shfl_sync(RLAP_FULL_MASK, nb, k);
+                const int knfill = __shfl_sync(RLAP_FULL_MASK, nfill, k);
+                const long long kslot0 = __shfl_sync(RLAP_FULL_MASK, slot0, k);
+                const int knslots = __shfl_sync(RLAP_FULL_MASK, nslots, k);
+                const int kM = __shfl_sync(RLAP_FULL_MASK, M, k);
+                eliminate_star_regs(P, rc, kidx, kb, knb, fbuf + k * FCAP, knfill, kslot0, knslots, kM, ls, pend, la);
+            }
             pend.flush(la);
             __syncwarp();
         }
@@ -1330,7 +1294,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
     const ModeParams<OV, ON, FULL>& P = tab.g[tab.bg[blockIdx.x]];
     extern __shared__ __align__(16) uint64_t smem[];
     __shared__ CtaScratch cs;
-    __shared__ int s_next, s_nsel;
+    __shared__ int s_nsel;
     __shared__ unsigned int s_lowbuf[ELIM_WARPS][LOWBUF];
     __shared__ LocalStats s_stats[ELIM_WARPS];
     const long long tid = (long long)((int)blockIdx.x - P.gblock0) * blockDim.x + threadIdx.x;   // inside the view group
@@ -1525,7 +1489,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
 #ifdef RLAP_DEBUG
             const int items_dbg = wl_end - wl_start;
 #endif
-            run_warp_items(P, rc, smem, &cs, &s_next, wl_start, wl_end, ls, la);
+            run_warp_items(P, rc, smem, &cs, wl_start, wl_end, ls, la);
             wl_start = wl_end;
             gsync(ST_T_D1);
             // stars too large for a lane or a register tile: the block-sized ones first (a block per star), then every
@@ -1559,7 +1523,6 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
         // live counter was seen crossing from above lvl to lvl or below by the elimination phase). While the low
         // list of a segment has an entry in play the bucket is taken from the list alone.
         constexpr int SEG_SM = 1024, WBUF = 224, MBUF = 160;
-        constexpr int LVL_AHEAD = RLAP_LVL_AHEAD;
         const int INF = 0x7fffffff;
         // (round, key) snapshots written by phase A, read by the bucket test of phase B; the emission's row offsets
         // are not needed before the elimination is over
@@ -1876,12 +1839,9 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
                 la.push(keep, idx);
             }
             dlap(1);
-            // B2: full scan of the segments that rescan. The level moves LVL_AHEAD keys past the bucket key found and
-            // the scan lists the vertices between the bucket and the level as well (they are "in play" from the next
-            // round on): the segment rescans again only when all those keys have drained, i.e. 1 + LVL_AHEAD times less
-            // often; the bucket of a round is still the minimum key alone (DESIGN.md §3.4 unchanged). LVL_AHEAD = 0 by default.
+            // B2: full scan of the segments that rescan; their level becomes the bucket key the scan found
             for (long long q = tid; q < VG; q += nthr) {
-                if (ldcg_i32(mkl + q) == INF) { const int m2 = ldcg_i32(mks + q); if (m2 != INF) P.lvl[q] = m2 + LVL_AHEAD; }
+                if (ldcg_i32(mkl + q) == INF) { const int m2 = ldcg_i32(mks + q); if (m2 != INF) P.lvl[q] = m2; }
             }
             {
                 const unsigned total = nselB * un;
@@ -1928,7 +1888,6 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
                         const unsigned mm = __ballot_sync(RLAP_FULL_MASK, member);
                         if (member) mbuf[mfill + __popc(mm & lt)] = idx;
                         mfill += __popc(mm);
-                        la.push(alive && key > m && key <= m + LVL_AHEAD, idx);
                     }
                     __syncwarp();
                     while (mfill >= 32) { mfill -= 32; test_members(mfill, 32); }
@@ -2034,7 +1993,7 @@ __global__ void __launch_bounds__(ELIM_THREADS, mode_ctas(OV, ON, FULL)) k_elimi
 #ifdef RLAP_DEBUG
             const int items_dbg = wl_end - wl_start;
 #endif
-            run_warp_items(P, rc, smem, &cs, &s_next, wl_start, wl_end, ls, la);
+            run_warp_items(P, rc, smem, &cs, wl_start, wl_end, ls, la);
             wl_start = wl_end;
             la.flush();
             gsync(ST_T_D1);

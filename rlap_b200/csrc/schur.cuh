@@ -44,7 +44,7 @@ enum {
     CTR_OVF0 = 9,        // degree mode: some segment selected more candidates than it may remove
     CTR_OVF1 = 10,
     CTR_ROUNDS = 11,
-    CTR_EMIT_C0 = 12,    // emission: tails of the six size-class lists (12..17; the elimination is over by then)
+    CTR_EMIT_C0 = 12,    // emission: tails of the seven size-class lists (12..18; the elimination is over by then)
     CTR_LOW0 = 14,       // degree mode: low-list tails, by round parity
     CTR_LOW1 = 15,
     CTR_LOWOVF0 = 16,    // degree mode: the low list of that parity overflowed (every segment rescans)

@@ -1,6 +1,6 @@
 // star.cuh — star staging shared by the elimination and emission kernels: shared-memory buffers,
 // sort + multi-edge merge of a staged star, and the register-resident (warp shuffle) variants used
-// for stars of at most 32 entries.
+// for stars of at most 32 entries, one star per warp and one entry per lane.
 #pragma once
 #include "rlap_device.cuh"
 #include "schur.cuh"
@@ -10,15 +10,6 @@ namespace rlap {
 
 __device__ __forceinline__ void set_status(const SchurParams& P, int code) { atomicCAS(P.ctr + CTR_STATUS, 0, code); }
 
-__device__ __forceinline__ StarBuf warp_buf(uint64_t* smem) {
-    int w = threadIdx.x >> 5;
-    StarBuf sb;
-    sb.A = smem + (size_t)w * 3 * CAP_WARP;
-    sb.Q = sb.A + CAP_WARP;
-    sb.K = sb.Q + CAP_WARP;
-    sb.cap = CAP_WARP;
-    return sb;
-}
 __device__ __forceinline__ StarBuf cta_buf(uint64_t* smem) {
     StarBuf sb;
     sb.A = smem;
@@ -201,10 +192,10 @@ __device__ __forceinline__ uint64_t warp_sort_u64(uint64_t a) {
 }
 
 // Merge the runs of equal neighbour of a SORTED register star (a = PAD beyond the entries).
-// On return: head lanes hold the merged entry (a with the merged fp32 weight, *q = summed fixed-point
-// weight), the other entries are marked dead (weight word RLAP_DEAD_W, *q = 0). Returns the head mask.
-// need_q: compute *q even when the star has no multi-edge (the elimination needs it, the emission does not).
-__device__ __forceinline__ unsigned warp_merge_sorted(uint64_t& a, unsigned long long& q, int& shift, bool need_q) {
+// On return every entry has its fixed-point weight *q, and head lanes hold the merged entry (a with the merged fp32
+// weight, *q = summed fixed-point weight, *mult = run length); the other entries are marked dead (weight word
+// RLAP_DEAD_W, *q = 0) and keep *mult = 1 (0 for padding). Returns the head mask.
+__device__ __forceinline__ unsigned warp_merge_sorted(uint64_t& a, unsigned long long& q, int& shift, int& mult) {
     const int lane = threadIdx.x & 31;
     const bool valid = a != RLAP_PAD_A;
     const uint32_t nb = a_nbr(a);
@@ -214,17 +205,14 @@ __device__ __forceinline__ unsigned warp_merge_sorted(uint64_t& a, unsigned long
     const unsigned hmask = __ballot_sync(RLAP_FULL_MASK, head);
     q = 0;
     shift = 0;
+    mult = valid ? 1 : 0;
     if (vmask == 0) return 0;
-    const bool dups = hmask != vmask;
-    if (dups || need_q) {
-        uint32_t wb = valid ? (uint32_t)a : 0u;
-        uint32_t wmaxb = warp_max_u32(wb);
-        shift = star_shift(__uint_as_float(wmaxb), __popc(vmask));
-        q = valid ? quantize(a_w(a), shift) : 0ull;
-    }
-    if (dups) {
+    const uint32_t wmaxb = warp_max_u32(valid ? (uint32_t)a : 0u);
+    shift = star_shift(__uint_as_float(wmaxb), __popc(vmask));
+    q = valid ? quantize(a_w(a), shift) : 0ull;
+    if (hmask != vmask) {
         unsigned long long qs = q;
-        int cnt = valid ? 1 : 0;
+        int cnt = mult;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) {
             unsigned long long oq = __shfl_down_sync(RLAP_FULL_MASK, qs, d);
@@ -235,6 +223,7 @@ __device__ __forceinline__ unsigned warp_merge_sorted(uint64_t& a, unsigned long
         }
         if (head) {
             q = qs;
+            mult = cnt;
             if (cnt > 1) a = ((uint64_t)nb << 32) | (uint64_t)__float_as_uint(dequantize_merged(qs, shift));
         } else if (valid) {
             q = 0;
@@ -244,21 +233,22 @@ __device__ __forceinline__ unsigned warp_merge_sorted(uint64_t& a, unsigned long
     return hmask;
 }
 
-
-// ascending bitonic sort of (k, a) pairs, one per lane, with payload q
-__device__ __forceinline__ void warp_sort_kaq(uint64_t& k, uint64_t& a, unsigned long long& q) {
+// ascending bitonic sort of (k, t, a) triples, one per lane, with payload q
+__device__ __forceinline__ void warp_sort_ktaq(uint64_t& k, uint64_t& t, uint64_t& a, unsigned long long& q) {
     const int lane = threadIdx.x & 31;
 #pragma unroll
     for (int kk = 2; kk <= 32; kk <<= 1) {
 #pragma unroll
         for (int j = kk >> 1; j > 0; j >>= 1) {
             uint64_t ok = __shfl_xor_sync(RLAP_FULL_MASK, k, j);
+            uint64_t ot = __shfl_xor_sync(RLAP_FULL_MASK, t, j);
             uint64_t oa = __shfl_xor_sync(RLAP_FULL_MASK, a, j);
             unsigned long long oq = __shfl_xor_sync(RLAP_FULL_MASK, q, j);
             bool take_min = (((lane & j) == 0) == ((lane & kk) == 0));
-            bool lt = (k < ok) || (k == ok && a < oa);
+            bool lt = (k != ok) ? (k < ok) : ((t != ot) ? (t < ot) : (a < oa));
             bool keep = (take_min == lt);
             k = keep ? k : ok;
+            t = keep ? t : ot;
             a = keep ? a : oa;
             q = keep ? q : oq;
         }
@@ -278,7 +268,6 @@ __device__ __forceinline__ int warp_upper_bound(unsigned long long C, int L, uns
     }
     return lo;
 }
-
 
 // ---------------------------------------------------------------------------------------------
 // a warp sorts 32 * R keys held in registers: element e = r * 32 + lane. Compare-exchange partners at
@@ -318,142 +307,5 @@ __device__ __forceinline__ void warp_sort_regs(uint64_t (&a)[R]) {
         }
     }
 }
-
-// ---------------------------------------------------------------------------------------------
-// sub-warp tiles: W lanes (8, 16 or 32) hold one star; 32 / W stars per warp run in lock step
-// ---------------------------------------------------------------------------------------------
-template <int W> struct Tile {
-    static __device__ __forceinline__ int tl() { return (int)(threadIdx.x & (W - 1)); }
-    static __device__ __forceinline__ int tbase() { return (int)(threadIdx.x & 31 & ~(W - 1)); }
-    static __device__ __forceinline__ unsigned low() { return W == 32 ? 0xffffffffu : ((1u << W) - 1u); }
-    static __device__ __forceinline__ unsigned ballot(bool pred) {
-        return (__ballot_sync(RLAP_FULL_MASK, pred) >> tbase()) & low();
-    }
-    static __device__ __forceinline__ uint64_t sort_u64(uint64_t a) {
-        const int l = tl();
-#pragma unroll
-        for (int k = 2; k <= W; k <<= 1) {
-#pragma unroll
-            for (int j = k >> 1; j > 0; j >>= 1) {
-                uint64_t o = __shfl_xor_sync(RLAP_FULL_MASK, a, j, W);
-                bool take_min = (((l & j) == 0) == ((l & k) == 0));
-                bool lt = a < o;
-                a = (take_min == lt) ? a : o;
-            }
-        }
-        return a;
-    }
-    static __device__ __forceinline__ void sort_kaq(uint64_t& k, uint64_t& a, unsigned long long& q) {
-        const int l = tl();
-#pragma unroll
-        for (int kk = 2; kk <= W; kk <<= 1) {
-#pragma unroll
-            for (int j = kk >> 1; j > 0; j >>= 1) {
-                uint64_t ok = __shfl_xor_sync(RLAP_FULL_MASK, k, j, W);
-                uint64_t oa = __shfl_xor_sync(RLAP_FULL_MASK, a, j, W);
-                unsigned long long oq = __shfl_xor_sync(RLAP_FULL_MASK, q, j, W);
-                bool take_min = (((l & j) == 0) == ((l & kk) == 0));
-                bool lt = (k < ok) || (k == ok && a < oa);
-                bool keep = (take_min == lt);
-                k = keep ? k : ok;
-                a = keep ? a : oa;
-                q = keep ? q : oq;
-            }
-        }
-    }
-    // same with a secondary key t between k and a
-    static __device__ __forceinline__ void sort_ktaq(uint64_t& k, uint64_t& t, uint64_t& a, unsigned long long& q) {
-        const int l = tl();
-#pragma unroll
-        for (int kk = 2; kk <= W; kk <<= 1) {
-#pragma unroll
-            for (int j = kk >> 1; j > 0; j >>= 1) {
-                uint64_t ok = __shfl_xor_sync(RLAP_FULL_MASK, k, j, W);
-                uint64_t ot = __shfl_xor_sync(RLAP_FULL_MASK, t, j, W);
-                uint64_t oa = __shfl_xor_sync(RLAP_FULL_MASK, a, j, W);
-                unsigned long long oq = __shfl_xor_sync(RLAP_FULL_MASK, q, j, W);
-                bool take_min = (((l & j) == 0) == ((l & kk) == 0));
-                bool lt = (k != ok) ? (k < ok) : ((t != ot) ? (t < ot) : (a < oa));
-                bool keep = (take_min == lt);
-                k = keep ? k : ok;
-                t = keep ? t : ot;
-                a = keep ? a : oa;
-                q = keep ? q : oq;
-            }
-        }
-    }
-    static __device__ __forceinline__ uint32_t max_u32(uint32_t v) {
-#pragma unroll
-        for (int d = W / 2; d > 0; d >>= 1) v = max(v, __shfl_xor_sync(RLAP_FULL_MASK, v, d, W));
-        return v;
-    }
-    static __device__ __forceinline__ unsigned long long incl_scan(unsigned long long v) {
-        const int l = tl();
-#pragma unroll
-        for (int d = 1; d < W; d <<= 1) {
-            unsigned long long t = __shfl_up_sync(RLAP_FULL_MASK, v, d, W);
-            if (l >= d) v += t;
-        }
-        return v;
-    }
-    // first tile-lane index in [0, L) whose C exceeds r (L if none)
-    static __device__ __forceinline__ int upper_bound(unsigned long long C, int L, unsigned long long r) {
-        int lo = 0, hi = L;
-        constexpr int ITERS = (W == 32 ? 6 : W == 16 ? 5 : 4);
-#pragma unroll
-        for (int it = 0; it < ITERS; it++) {
-            int mid = (lo + hi) >> 1;
-            unsigned long long cm = __shfl_sync(RLAP_FULL_MASK, C, mid & (W - 1), W);
-            if (lo < hi) {
-                if (cm > r) hi = mid; else lo = mid + 1;
-            }
-        }
-        return lo;
-    }
-    // merge runs of equal neighbour of a sorted tile star; see warp_merge_sorted
-    static __device__ __forceinline__ unsigned merge_sorted(uint64_t& a, unsigned long long& q, int& shift, bool need_q,
-                                                            int& mult) {
-        const int l = tl();
-        const bool valid = a != RLAP_PAD_A;
-        const uint32_t nb = a_nbr(a);
-        const uint32_t pnb = __shfl_up_sync(RLAP_FULL_MASK, nb, 1, W);
-        const bool head = valid && (l == 0 || pnb != nb);
-        const unsigned vmask = ballot(valid);
-        const unsigned hmask = ballot(head);
-        q = 0;
-        shift = 0;
-        mult = valid ? 1 : 0;
-        const bool dups = hmask != vmask;
-        const bool anyd = __any_sync(RLAP_FULL_MASK, dups);   // keep the tiles of a warp in lock step
-        uint32_t wmaxb = max_u32(valid ? (uint32_t)a : 0u);
-        if (vmask != 0 && (dups || need_q)) {
-            shift = star_shift(__uint_as_float(wmaxb), __popc(vmask));
-            q = valid ? quantize(a_w(a), shift) : 0ull;
-        }
-        if (anyd) {
-            unsigned long long qs = q;
-            int cnt = valid ? 1 : 0;
-#pragma unroll
-            for (int d = 1; d < W; d <<= 1) {
-                unsigned long long oq = __shfl_down_sync(RLAP_FULL_MASK, qs, d, W);
-                int oc = __shfl_down_sync(RLAP_FULL_MASK, cnt, d, W);
-                uint32_t onb = __shfl_down_sync(RLAP_FULL_MASK, nb, d, W);
-                bool ov = (l + d < W) && ((vmask >> ((l + d) & (W - 1))) & 1u);
-                if (dups && valid && ov && onb == nb) { qs += oq; cnt += oc; }
-            }
-            if (dups) {
-                if (head) {
-                    q = qs;
-                    mult = cnt;
-                    if (cnt > 1) a = ((uint64_t)nb << 32) | (uint64_t)__float_as_uint(dequantize_merged(qs, shift));
-                } else if (valid) {
-                    q = 0;
-                    a = ((uint64_t)nb << 32) | (uint64_t)RLAP_DEAD_W;
-                }
-            }
-        }
-        return hmask;
-    }
-};
 
 }  // namespace rlap

@@ -23,7 +23,7 @@ from dataclasses import dataclass, field
 import numpy as np
 
 LCAP, LANE_NB_MAX = 16, 48               # schur.cu eliminate_star_lane
-TILE_MAX, FCAP = 32, 16                  # schur.cu run_warp_items: register tiles
+TILE_MAX, FCAP = 32, 16                  # schur.cu run_warp_items: register tiles (eliminate_star_regs)
 CAP_WARP, STAGE_CAP, HUB_DEG = 128, 128, 64   # schur.cuh
 ELIM_CAP_CTA = 1024                      # schur.cuh: CAP_WARP x 8 warps of the elimination block
 FS_LANE, FS_NB_MAX, FSORT_MAX = 16, 40, 32    # emit.cu k_emit_fsort
@@ -245,9 +245,9 @@ TIERS = [
      lambda q: not q["prot"] and _lane(q) and q["multi"] != "none", _NOT_FULL),
     ("elim", "lane_to_smem_key_tie", "schur.cu eliminate_star_lane: tie |= ky == kx",
      lambda q: not q["prot"] and _lane(q) and q["tie"] and _shuffle(q), _SHUF),
-    ("elim", "tile", "schur.cu run_warp_items K_TILE / run_tier<32>",
+    ("elim", "tile", "schur.cu run_warp_items K_TILE / eliminate_star_regs",
      lambda q: not q["prot"] and _tile(q), _ALL),
-    ("elim", "tile_key_tie", "schur.cu run_tier<32> with a 32-bit shuffle-key tie",
+    ("elim", "tile_key_tie", "schur.cu eliminate_star_regs with a 32-bit shuffle-key tie",
      lambda q: not q["prot"] and _tile(q) and q["tie"] and _shuffle(q), _SHUF),
     ("elim", "warp_smem", "schur.cu run_warp_items K_SMEM / run_smem_items",
      lambda q: not q["prot"] and _warp_smem(q), _ALL),
@@ -260,7 +260,7 @@ TIERS = [
      [(ov, on, False) for ov, on in MODES if ov == "random"]),
     ("elim", "lane_lv16", "schur.cu run_warp_items: the largest lane star, lv = LCAP",
      lambda q: not q["prot"] and _lane(q) and q["lv"] == LCAP and q["multi"] == "none", _NOT_FULL),
-    ("elim", "tile_lv17", "schur.cu run_warp_items: the smallest tile after the lane stars, lv = LCAP + 1",
+    ("elim", "tile_lv17", "schur.cu eliminate_star_regs: the smallest tile after the lane stars, lv = LCAP + 1",
      lambda q: not q["prot"] and _tile(q) and q["lv"] == LCAP + 1, _NOT_FULL),
     ("elim", "block", "schur.cu run_block_items, lv <= ELIM_CAP_CTA",
      lambda q: not q["prot"] and CAP_WARP < q["lv"] <= ELIM_CAP_CTA, _ALL),
@@ -295,7 +295,7 @@ TIERS = [
     ("emit", "merge_fill_base_warp", "emit.cu k_emit_fsort warp: a fill parallel to a base edge",
      lambda q: q["prot"] and q["multi"] == "fill_base" and FS_LANE < q["fills"] <= FSORT_MAX, _NOT_FULL),
 ] + [
-    ("emit", f"merge_class_{lv}", "emit.cu size_class / k_emit_sort_*",
+    ("emit", f"merge_class_{lv}", "emit.cu size_class / k_emit_sort_mid<R>, k_emit_sort_block, k_emit_sort_big",
      (lambda lv: lambda q: q["prot"] and q["multi"] != "none" and q["lv"] == lv)(lv), _NOT_FULL)
     for lv in (32, 33, 64, 65, 128, 129, 256, 257, 512, 513, 2048, 2049, 12288, 12289)
 ] + [
